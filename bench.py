@@ -2,9 +2,9 @@
 """
 bench.py -- monoloco hot path on B200:  detections/s of the fused forward (pre-process -> LocoModel -> decode).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
-Contract (see the task statement / DESIGN.md §6):
+What it reports (DESIGN.md §6):
   * one step = one pass of the hot path over one batch of synthetic 17-keypoint detections
     (BASELINE.json configs[1]: LocoModel mono 34->9, 3 stages x 1024, batch 4096 per GPU, fp32);
   * `value`  = whole-job detections/s with inputs resident in HBM, timed with CUDA events on the launching stream,
@@ -12,6 +12,9 @@ Contract (see the task statement / DESIGN.md §6):
   * `e2e`    = same metric through the public host-buffer call (pinned host memory; H2D + kernel(+ all-gather) + D2H
                per step): `mlb_forward_host` at N = 1, `ShardedLoco.forward_host` at N > 1;
   * `roofline` (binding bound first), `cpu_baseline`, `clocks`, `gpu_launches` as specified.
+  * --dump-outputs DIR: after the timed steps, the arrays the last timed step handed its caller, as DIR/<name>.npy in
+    float32 (`raw` [B,9] and `dec` [B,8] at N = 1, the gathered `rows` [N*B,20] at N > 1, `raw` for --impl reference).
+    Inputs are seeded, so two builds run with the same arguments can be compared file for file.
   * --impl reference: the reference's CPU implementation of the path (oracle/torch_port.py = the same torch-eager
     op sequence as the reference nn.Module) timed on the host cores.
 Multi-GPU: launched by torch.distributed.run; detections shard over ranks (weak scaling, 4096 per GPU); the step is ONE
@@ -33,6 +36,25 @@ import torch  # noqa: E402
 
 METRIC = "detections/sec LocoModel(34->9, 3x1024) fused forward @ batch 4096 per GPU"
 UNIT = "detections/s"
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor or array} as path/<name>.npy in float32.  All arrays share the row dimension; when they come to
+    more than DUMP_BYTES, the same fixed, seeded sample of rows is kept from each and its row numbers go to row_index.npy
+    (float64), so that two runs with the same arguments write the same rows."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: (v.detach().cpu().numpy() if torch.is_tensor(v) else np.asarray(v)).astype(np.float32)
+              for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[:1].nbytes for a in arrays.values())
+    if n * row_bytes > DUMP_BYTES:
+        k = (DUMP_BYTES - 4096) // (row_bytes + 8)   # 4 KiB for the .npy headers, 8 B per row for its index
+        idx = np.sort(np.random.RandomState(0).choice(n, k, replace=False))
+        arrays = {name: a[idx] for name, a in arrays.items()}
+        arrays['row_index'] = idx.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
 
 
 def profile_json(name):
@@ -328,6 +350,8 @@ def run_reference(args, rank, world):
             O.extract_outputs(out.numpy())                             # process.py:231-278
             if i >= args.warmup:
                 times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {'raw': out})
     ms = 1e3 * float(np.mean(times))
     val = B / (ms * 1e-3)
     line = {"impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -381,7 +405,11 @@ def main():
     ap.add_argument('--rows-per-group', type=int, default=0)
     ap.add_argument('--gather', default='fused', choices=['fused', 'nccl'],
                     help='multi-GPU output all-gather: fused peer stores + device-side flags, or NCCL')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get('RANK', '0'))
@@ -440,7 +468,7 @@ def main():
         for e0, e1 in ev:
             flush.zero_()
             e0.record(st)
-            step()
+            out = step()
             e1.record(st)
         torch.cuda.synchronize(dev)
         launches = lib.mlb_launch_count() - launches0
@@ -449,6 +477,9 @@ def main():
             torch.cuda.synchronize(dev)
     eng.check_error()
     eng.last_kernel_of_step = eng.last_kernel()
+    # before the all-reduce below: at N > 1 the rows are a view of a gather buffer that every rank's next step overwrites
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out if sharded is None else {'rows': out})
     per_step = torch.tensor([e0.elapsed_time(e1) for e0, e1 in ev], dtype=torch.float64, device=dev)
     total = per_step.sum().reshape(1)
     if world > 1:
