@@ -102,6 +102,8 @@ enum { MLB_IN_X = 0,          /* pre-processed network input [B, input_size] (nn
        MLB_IN_KPS = 1,        /* raw keypoints [B,3,17] (u,v,conf rows): process.py:47-67 fused      */
        MLB_IN_KPS_STEREO = 2  /* left [L,3,17] + right [R,3,17], all-vs-all rows l*R+r: :25-44 fused */ };
 
+/* At most one MLB_FWD_FORCE_* may be set, and it must name a kernel this handle has for this many rows (otherwise
+ * mlb_forward fails).  A forced kernel ignores rows_per_group. */
 enum { MLB_FWD_ZERO_CENTER = 1, /* preprocess_monoloco(zero_center=True) (net.py:96, legacy)        */
        MLB_FWD_DROPOUT     = 2, /* MC-dropout pass: top-level dropout sites active (net.py:141)     */
        MLB_FWD_RES_TMEM    = 4, /* stash the residual x of MyLinearSimple in Tensor Memory (default) */

@@ -12,7 +12,7 @@ LIB_DIR = os.path.join(HERE, 'lib')
 OBJ_DIR = os.path.join(LIB_DIR, 'obj')
 LIB_PATH = os.path.join(LIB_DIR, 'libmonoloco_b200.so')
 HEADER = os.path.join(HERE, '..', 'include', 'monoloco_b200.h')
-SOURCES = ['forward.cu', 'forward_small.cu', 'forward_wide.cu', 'forward_wide2.cu', 'train.cu', 'optim.cu', 'post.cu', 'probe_tc.cu', 'forward_tc.cu']
+SOURCES = ['model.cu', 'forward.cu', 'forward_small.cu', 'forward_wide.cu', 'forward_wide2.cu', 'train.cu', 'optim.cu', 'post.cu', 'probe_tc.cu', 'forward_tc.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-std=c++17', '-Xcompiler', '-fPIC']
 
 

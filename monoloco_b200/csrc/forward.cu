@@ -23,15 +23,9 @@
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
-#include <stdio.h>
-#include <stdlib.h>
 #include <string.h>
 
-#include <atomic>
-#include <mutex>
-#include <string>
-
-#include "fwd_common.cuh"
+#include "fwd_family.cuh"
 
 namespace mlb {
 
@@ -425,9 +419,6 @@ __global__ void __launch_bounds__(MAX_THREADS, 1) loco_forward_kernel(const __gr
     if (res_tmem && warp == 0) tmem_dealloc(*tmem_slot, tmem_cols);
 }
 
-// a rank whose shard is empty still takes part in the completion protocol of the fused all-gather
-__global__ void gather_flag_only_kernel(const __grid_constant__ FwdParams p) { gather_finish(p); }
-
 // ------------------------------------------------------------------------------------------------
 // stand-alone pre-process (process.py:47-67) for callers that never run the network
 // ------------------------------------------------------------------------------------------------
@@ -538,342 +529,25 @@ __global__ void __launch_bounds__(512) ffma2_probe_kernel(int iters, float* sink
 }  // namespace mlb
 
 // ================================================================================================
-// host side: C ABI
+// host side: the row-tile family and the stand-alone entry points
 // ================================================================================================
 using namespace mlb;
 
-// forward_small.cu
-size_t mlb_small_smem_bytes(int L);
-cudaError_t mlb_small_pack(const float* blob, const mlb_op* ops, int n_ops, int L, float* slab, long long* slab_off, cudaStream_t st);
-cudaError_t mlb_small_launch(const FwdParams& p, const float* slab, const long long* slab_off, int n_clusters, cudaStream_t st);
-int mlb_small_max_clusters(int L);
-// forward_wide2.cu
-size_t mlb_wide2_slab_floats(const mlb_op* ops, int n_ops, int L, long long* slab_off);
-cudaError_t mlb_wide2_pack(const float* blob, const mlb_op* ops, int n_ops, int L, float* slab, const long long* slab_off, cudaStream_t st);
-bool mlb_wide2_supported(const mlb_op* ops, int n_ops, int L, int out_size, int n_sms);
-int mlb_wide2_epochs(const mlb_op* ops, int n_ops);
-size_t mlb_wide2_xg_pairs(int L);
-size_t mlb_wide2_hg_pairs(int L);
-cudaError_t mlb_wide2_set_marks(unsigned long long* ptr);
-cudaError_t mlb_wide2_launch(const FwdParams& p, const float* wslab, const long long* wslab_off, unsigned long long* xg,
-                             unsigned long long* hg, unsigned epoch_base, cudaStream_t st);
-// forward_tc.cu
-struct mlb_tc_state;
-bool mlb_tc_supported(int L);
-mlb_tc_state* mlb_tc_prepare(const float* blob_dev, const mlb_op* ops, int n_ops, int L, cudaStream_t st, cudaError_t* err);
-cudaError_t mlb_tc_repack(mlb_tc_state* t, const float* blob_dev, const mlb_op* ops, int n_ops, int L, cudaStream_t st);
-void mlb_tc_free(mlb_tc_state* t);
-int mlb_tc_clusters(const mlb_tc_state* t, int n_rows);
-cudaError_t mlb_tc_launch(const mlb_tc_state* t, const FwdParams& p, cudaStream_t st);
-cudaError_t mlb_tc_set_marks(unsigned long long* ptr);
-int mlb_tc_max_clusters(const mlb_tc_state* t);
-// forward_wide.cu
-size_t mlb_wide_slab_floats(const mlb_op* ops, int n_ops, int L, long long* slab_off);
-cudaError_t mlb_wide_pack(const float* blob, const mlb_op* ops, int n_ops, int L, float* slab, const long long* slab_off, cudaStream_t st);
-bool mlb_wide_supported(int L, int n_sms);
-int mlb_wide_barriers(const mlb_op* ops, int n_ops);
-cudaError_t mlb_wide_set_marks(unsigned long long* ptr);
-cudaError_t mlb_wide_launch(const FwdParams& p, const float* wslab, const long long* wslab_off, float* xg, unsigned* bar,
-                            unsigned bar_base, cudaStream_t st);
+cudaError_t TileFamily::set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_fwd_marks, &ptr, sizeof(ptr)); }
 
-struct mlb_model {
-    mlb_model_desc desc;
-    mlb_op ops[MLB_MAX_OPS];
-    int device;
-    int n_sms;
-    float* blob_dev;
-    size_t n_floats;
-    float* slab_dev;               // slab-major W^T copies for the small-batch cluster kernel (L == 1024 only)
-    long long slab_off[MLB_MAX_OPS];
-    int small_conc;                // co-resident 8-CTA clusters (cudaOccupancyMaxActiveClusters)
-    float* wslab_dev;              // per-CTA column slabs for the whole-grid latency kernel (forward_wide.cu), or null
-    long long wslab_off[MLB_MAX_OPS];
-    float* wide_xg;                // [2][L][32] inter-CTA exchange tiles
-    unsigned* wide_bar;            // monotonic grid-barrier counter
-    unsigned wide_bar_count;       // host copy of the counter after the launches issued so far
-    bool wide_disabled;            // a cooperative launch was refused once: stay on the other kernels
-    float* w2slab_dev;             // [cluster][K slice] slabs for the second-generation latency kernel (forward_wide2.cu), or null
-    long long w2slab_off[MLB_MAX_OPS];
-    unsigned long long* wide2_xg;  // (value, epoch) exchange pairs
-    unsigned long long* wide2_hg;  // head partial pairs
-    unsigned wide2_epoch;          // epochs consumed by the launches issued so far
-    bool wide2_disabled;
-    float* res_scratch;
-    size_t res_floats;
-    mlb_tc_state* tc;              // tensor-core kernel state (weight planes, cluster workspace), or null
-    int last_kernel;               // MLB_KERNEL_* of the most recent mlb_forward launch
-    // per-wave times measured on this device at mlb_create (ms): FFMA cluster wave, row-tile wave = a + b * TM, tensor-core wave
-    double t_cluster_wave, t_tile_a, t_tile_b, t_tc_wave;
-    bool calibrated;
-    bool ffma_ok;                  // the FFMA kernels fit this width (L <= 1024)
-    int tc_min_rows;               // batches of at least this many rows go to the tensor-core kernel
-    unsigned* gather_done;         // monotonic count of CTAs that finished their peer stores (fused all-gather)
-    unsigned gather_done_count;    // host copy of the value it reaches after the launches issued so far
-    int* err_flag_dev;             // device view of err_flag_host
-    int* err_flag_host;            // mapped pinned host word: the host reads it after a sync without a copy
-    // staging for mlb_forward_host
-    float* st_in;
-    float* st_in_r;
-    float* st_raw;
-    float* st_dec;
-    float* st_xyzc;
-    float* st_x;
-    size_t st_rows;
-    size_t st_rows_r;
-    bool attr_set;
-};
+bool TileFamily::covers(int L) { return L >= 128 && L <= 1024 && (L % 128) == 0; }
 
-thread_local std::string g_mlb_err;  // shared with train.cu
-#define g_err g_mlb_err
-static std::atomic<uint64_t> g_launches{0};
-void mlb_count_launch() { g_launches++; }
-
-static int fail(const std::string& msg) {
-    g_err = msg;
-    return -1;
-}
-#define CU(call)                                                                                   \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess) return fail(std::string(#call) + ": " + cudaGetErrorString(e_));   \
-    } while (0)
-
-extern "C" const char* mlb_last_error(void) { return g_err.c_str(); }
-extern "C" int mlb_abi_version(void) { return MLB_ABI_VERSION; }
-extern "C" uint64_t mlb_launch_count(void) { return g_launches.load(); }
-
-// profiling aid: point the tile kernel's timestamp marks at a device buffer of >= 4 * n_ops + 4 uint64 (nullptr: off).
-// CTA 0 stamps: [0] start, [1] input tile staged, per op i [2+4i] GEMM done, [3+4i] epilogue math done, [4+4i] CTA
-// synchronised, [5+4i] activation tile rewritten; [2+4n] heads done, [3+4n] rows stored.
-extern "C" int mlb_debug_fwd_marks(void* dev_buf) {
-    unsigned long long* ptr = reinterpret_cast<unsigned long long*>(dev_buf);
-    cudaError_t e = cudaMemcpyToSymbol(mlb::g_fwd_marks, &ptr, sizeof(ptr));
-    if (e == cudaSuccess) e = mlb_wide_set_marks(ptr);
-    if (e == cudaSuccess) e = mlb_tc_set_marks(ptr);
-    if (e == cudaSuccess) e = mlb_wide2_set_marks(ptr);
-    if (e != cudaSuccess) {
-        g_mlb_err = std::string("mlb_debug_fwd_marks: ") + cudaGetErrorString(e);
-        return -1;
-    }
-    return 0;
-}
-extern "C" int mlb_num_sms(mlb_handle h) { return h ? h->n_sms : 0; }
-extern "C" int mlb_last_kernel(mlb_handle h) { return h ? h->last_kernel : -1; }
-extern "C" int mlb_tc_resident_clusters(mlb_handle h) { return (h && h->tc) ? mlb_tc_max_clusters(h->tc) : 0; }
-extern "C" int mlb_device_error(mlb_handle h) { return h ? *reinterpret_cast<volatile int*>(h->err_flag_host) : -1; }
-
-static size_t fwd_smem_bytes(int L) {
-    size_t fl = (size_t)L * MP + MP * OUT_LD + MP * 4 + (size_t)NSTAGE * KC * L;
-    return fl * sizeof(float) + 2 * NSTAGE * sizeof(uint64_t) + 16;
-}
-
-static void calibrate(mlb_handle h);
-static int pick_rows_per_group(int n_rows, int n_ctas);
-
-extern "C" int mlb_create(const mlb_model_desc* desc, const mlb_op* ops, const float* packed_host, size_t n_floats,
-                          int device, mlb_handle* out) {
-    if (!desc || !ops || !packed_host || !out) return fail("mlb_create: null argument");
-    if (desc->abi_version != MLB_ABI_VERSION) return fail("mlb_create: ABI version mismatch");
-    if (desc->n_ops < 1 || desc->n_ops > MLB_MAX_OPS) return fail("mlb_create: n_ops out of range");
-    const int L = desc->linear_size;
-    const bool ffma_ok = L >= 128 && L <= 1024 && (L % 128) == 0;
-    if (!ffma_ok && !mlb_tc_supported(L))
-        return fail("mlb_create: linear_size must be a multiple of 128 up to 1024 or a multiple of 256 up to 2048 "
-                    "(monoloco_b200.packing zero-pads other widths)");
-    if (desc->input_size < 1 || desc->input_size > 68) return fail("mlb_create: input_size must be in [1,68]");
-    if (desc->output_size < 1 || desc->output_size > OUT_LD) return fail("mlb_create: output_size must be in [1,16]");
-    for (int i = 0; i < desc->n_ops; ++i) {
-        const mlb_op& op = ops[i];
-        if (op.type == MLB_OP_GEMM) {
-            if (op.N != L) return fail("mlb_create: GEMM op width must equal linear_size");
-            if (op.Kpad % KC != 0 || op.Kpad < op.K) return fail("mlb_create: bad Kpad");
-            if ((op.flags & MLB_F_IN_XIN) ? (op.Kpad > KIN_MAX) : (op.K != L)) return fail("mlb_create: bad GEMM K");
-            if ((op.w_off % 4) || (op.scale_off % 4) || (op.shift_off % 4)) return fail("mlb_create: unaligned offsets");
-            if ((size_t)op.w_off + (size_t)op.Kpad * L > n_floats) return fail("mlb_create: weights out of blob");
-        } else if (op.type == MLB_OP_HEAD) {
-            if (op.K != L || (op.K % 4)) return fail("mlb_create: HEAD K must equal linear_size");
-            if (op.N < 1 || op.out_col < 0 || op.out_col + op.N > desc->output_size) return fail("mlb_create: bad HEAD columns");
-            if (op.w_off % 4) return fail("mlb_create: unaligned HEAD weights");
-            if ((size_t)op.w_off + (size_t)op.N * op.K > n_floats) return fail("mlb_create: head weights out of blob");
-        } else {
-            return fail("mlb_create: unknown op type");
-        }
-    }
-    CU(cudaSetDevice(device));
-    cudaDeviceProp prop;
-    CU(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) return fail("mlb_create: this library is built for sm_100a (B200) only");
-    mlb_model* m = new mlb_model();
-    memset(m, 0, sizeof(*m));
-    m->desc = *desc;
-    memcpy(m->ops, ops, sizeof(mlb_op) * desc->n_ops);
-    m->device = device;
-    m->n_sms = prop.multiProcessorCount;
-    m->n_floats = n_floats;
-    m->ffma_ok = ffma_ok;
-    CU(cudaMalloc(&m->blob_dev, n_floats * sizeof(float)));
-    CU(cudaMemcpy(m->blob_dev, packed_host, n_floats * sizeof(float), cudaMemcpyHostToDevice));
-    if (mlb_tc_supported(L)) {
-        cudaError_t et = cudaSuccess;
-        m->tc = mlb_tc_prepare(m->blob_dev, m->ops, desc->n_ops, L, 0, &et);
-        if (m->tc == nullptr) {
-            if (!ffma_ok) return fail(std::string("mlb_create: tensor-core kernel set-up: ") + cudaGetErrorString(et));
-            cudaGetLastError();  // the FFMA kernels cover this width: carry on without the tensor-core path
-        }
-        CU(cudaDeviceSynchronize());
-    }
-    if (L == 1024) {
-        size_t gemm_floats = 0;
-        for (int i = 0; i < desc->n_ops; ++i)
-            if (ops[i].type == MLB_OP_GEMM) gemm_floats += (size_t)ops[i].Kpad * L;
-        CU(cudaMalloc(&m->slab_dev, gemm_floats * sizeof(float)));
-        CU(mlb_small_pack(m->blob_dev, m->ops, desc->n_ops, L, m->slab_dev, m->slab_off, 0));
-        CU(cudaDeviceSynchronize());
-        m->small_conc = mlb_small_max_clusters(L);
-        if (m->small_conc < 1) m->small_conc = 8;
-    }
-    if (m->tc != nullptr) {
-        // When the tensor-core kernel takes over (measured, DESIGN.md §3): a wave of 128-row tiles takes ~0.32 ms whatever
-        // the batch.  One wave of 8-CTA FFMA clusters (16 rows each, `small_conc` co-resident) takes 0.18 ms, two take
-        // 0.36 ms: the cluster kernel keeps the batches that fit ONE wave.  Without the cluster kernel (L != 1024) a
-        // row-tile wave costs >= 0.9 ms, so everything beyond the whole-grid kernel's 64 rows goes to the tensor cores.
-        m->tc_min_rows = m->slab_dev != nullptr ? m->small_conc * 16 + 1 : 65;
-        if (getenv("MLB_TC_MIN_ROWS")) m->tc_min_rows = atoi(getenv("MLB_TC_MIN_ROWS"));
-    }
-    if (ffma_ok && mlb_wide_supported(L, m->n_sms)) {
-        const size_t wf = mlb_wide_slab_floats(m->ops, desc->n_ops, L, m->wslab_off);
-        CU(cudaMalloc(&m->wslab_dev, wf * sizeof(float)));
-        CU(mlb_wide_pack(m->blob_dev, m->ops, desc->n_ops, L, m->wslab_dev, m->wslab_off, 0));
-        CU(cudaMalloc(&m->wide_xg, (size_t)2 * L * 32 * sizeof(float)));
-        CU(cudaMemset(m->wide_xg, 0, (size_t)2 * L * 32 * sizeof(float)));
-        CU(cudaMalloc(&m->wide_bar, sizeof(unsigned)));
-        CU(cudaMemset(m->wide_bar, 0, sizeof(unsigned)));
-        m->wide_bar_count = 0;
-        CU(cudaDeviceSynchronize());
-    }
-    if (ffma_ok && !getenv("MLB_NO_WIDE2") && mlb_wide2_supported(m->ops, desc->n_ops, L, desc->output_size, m->n_sms)) {
-        const size_t wf = mlb_wide2_slab_floats(m->ops, desc->n_ops, L, m->w2slab_off);
-        CU(cudaMalloc(&m->w2slab_dev, wf * sizeof(float)));
-        CU(mlb_wide2_pack(m->blob_dev, m->ops, desc->n_ops, L, m->w2slab_dev, m->w2slab_off, 0));
-        CU(cudaMalloc(&m->wide2_xg, mlb_wide2_xg_pairs(L) * sizeof(unsigned long long)));
-        CU(cudaMemset(m->wide2_xg, 0, mlb_wide2_xg_pairs(L) * sizeof(unsigned long long)));
-        CU(cudaMalloc(&m->wide2_hg, mlb_wide2_hg_pairs(L) * sizeof(unsigned long long)));
-        CU(cudaMemset(m->wide2_hg, 0, mlb_wide2_hg_pairs(L) * sizeof(unsigned long long)));
-        CU(cudaDeviceSynchronize());
-    }
-    m->res_floats = (size_t)m->n_sms * 4 * 128 * 256;  // up to 4 resident CTAs per SM for narrow models
-    CU(cudaMalloc(&m->res_scratch, m->res_floats * sizeof(float)));
-    CU(cudaMalloc(&m->gather_done, sizeof(unsigned)));
-    CU(cudaMemset(m->gather_done, 0, sizeof(unsigned)));
-    CU(cudaHostAlloc(reinterpret_cast<void**>(&m->err_flag_host), sizeof(int), cudaHostAllocMapped));
-    *m->err_flag_host = 0;
-    CU(cudaHostGetDevicePointer(reinterpret_cast<void**>(&m->err_flag_dev), m->err_flag_host, 0));
-    calibrate(m);
-    *out = m;
-    return 0;
-}
-
-// Time one wave of every kernel family on THIS device (CUDA events, L2 warm, 2 launches each, the second one counts) so that
-// the batch-size thresholds of mlb_forward are measured quantities instead of constants from another box.  ~10 launches.
-static void calibrate(mlb_handle h) {
-    const mlb_model_desc& d = h->desc;
-    h->t_cluster_wave = 0.185, h->t_tile_a = 0.42, h->t_tile_b = 0.067, h->t_tc_wave = 0.33;  // round-2 B200 defaults
-    if (getenv("MLB_NO_CALIBRATE")) return;
-    const int max_rows = h->n_sms * 32;
-    float *x = nullptr, *raw = nullptr;
-    if (cudaMalloc(&x, (size_t)max_rows * d.input_size * sizeof(float)) != cudaSuccess) return;
-    if (cudaMalloc(&raw, (size_t)max_rows * d.output_size * sizeof(float)) != cudaSuccess) { cudaFree(x); return; }
-    cudaMemset(x, 0, (size_t)max_rows * d.input_size * sizeof(float));
-    cudaEvent_t e0, e1;
-    cudaEventCreate(&e0), cudaEventCreate(&e1);
-    auto time_one = [&](int rows, int flags, int tm) -> double {
-        mlb_forward_args a;
-        memset(&a, 0, sizeof(a));
-        a.input_kind = MLB_IN_X, a.flags = flags, a.n_rows = rows, a.rows_per_group = tm, a.x = x, a.out_raw = raw;
-        float ms = -1.f;
-        for (int rep = 0; rep < 2; ++rep) {
-            cudaEventRecord(e0, 0);
-            if (mlb_forward(h, &a, nullptr) != 0) return -1.0;
-            cudaEventRecord(e1, 0);
-            if (cudaEventSynchronize(e1) != cudaSuccess) return -1.0;
-            cudaEventElapsedTime(&ms, e0, e1);
-        }
-        return (double)ms;
-    };
-    if (h->ffma_ok) {
-        const double t8 = time_one(h->n_sms * 16, MLB_FWD_FORCE_TILE, 8), t16 = time_one(h->n_sms * 32, MLB_FWD_FORCE_TILE, 16);
-        if (t8 > 0 && t16 > t8) h->t_tile_b = (t16 - t8) / 8.0, h->t_tile_a = t8 - 8.0 * h->t_tile_b;
-        if (h->slab_dev != nullptr) {
-            const double tc = time_one(h->small_conc * 16, MLB_FWD_FORCE_CLUSTER, 0);
-            if (tc > 0) h->t_cluster_wave = tc;
-        }
-    }
-    if (h->tc != nullptr) {
-        const double tt = time_one(128, MLB_FWD_FORCE_TC, 0);
-        if (tt > 0) h->t_tc_wave = tt;
-    }
-    cudaEventDestroy(e0), cudaEventDestroy(e1);
-    cudaFree(x), cudaFree(raw);
-    cudaGetLastError();
-    h->calibrated = true;
-}
-
-extern "C" int mlb_kernel_times(mlb_handle h, double out_ms[4]) {
-    if (!h || !out_ms) return fail("mlb_kernel_times: null argument");
-    out_ms[0] = h->t_cluster_wave, out_ms[1] = h->t_tile_a, out_ms[2] = h->t_tile_b, out_ms[3] = h->t_tc_wave;
-    return h->calibrated ? 1 : 0;
-}
-
-extern "C" int mlb_update_weights(mlb_handle h, const float* packed_host, size_t n_floats, void* stream) {
-    if (!h || !packed_host) return fail("mlb_update_weights: null argument");
-    if (n_floats != h->n_floats) return fail("mlb_update_weights: blob size changed");
-    CU(cudaSetDevice(h->device));
-    CU(cudaMemcpyAsync(h->blob_dev, packed_host, n_floats * sizeof(float), cudaMemcpyHostToDevice, (cudaStream_t)stream));
-    if (h->slab_dev)
-        CU(mlb_small_pack(h->blob_dev, h->ops, h->desc.n_ops, h->desc.linear_size, h->slab_dev, h->slab_off, (cudaStream_t)stream));
-    if (h->wslab_dev)
-        CU(mlb_wide_pack(h->blob_dev, h->ops, h->desc.n_ops, h->desc.linear_size, h->wslab_dev, h->wslab_off, (cudaStream_t)stream));
-    if (h->w2slab_dev)
-        CU(mlb_wide2_pack(h->blob_dev, h->ops, h->desc.n_ops, h->desc.linear_size, h->w2slab_dev, h->w2slab_off, (cudaStream_t)stream));
-    if (h->tc) CU(mlb_tc_repack(h->tc, h->blob_dev, h->ops, h->desc.n_ops, h->desc.linear_size, (cudaStream_t)stream));
-    return 0;
-}
-
-extern "C" void mlb_destroy(mlb_handle h) {
-    if (!h) return;
-    cudaSetDevice(h->device);
-    cudaFree(h->blob_dev);
-    cudaFree(h->slab_dev);
-    cudaFree(h->wslab_dev);
-    cudaFree(h->wide_xg);
-    cudaFree(h->wide_bar);
-    cudaFree(h->w2slab_dev);
-    cudaFree(h->wide2_xg);
-    cudaFree(h->wide2_hg);
-    cudaFree(h->res_scratch);
-    cudaFree(h->gather_done);
-    mlb_tc_free(h->tc);
-    cudaFreeHost(h->err_flag_host);
-    cudaFree(h->st_in);
-    cudaFree(h->st_in_r);
-    cudaFree(h->st_raw);
-    cudaFree(h->st_dec);
-    cudaFree(h->st_xyzc);
-    cudaFree(h->st_x);
-    delete h;
-}
-
-static int pick_rows_per_group(int n_rows, int n_ctas) {
-    // minimise waves(tm) * tm  (time ~ rows per CTA per wave), prefer the larger tile on ties
-    int best = 16;
-    long best_cost = -1;
-    for (int tm = 16; tm >= 8; tm -= 2) {
-        const long tiles = (n_rows + 2 * tm - 1) / (2 * tm);
-        const long waves = (tiles + n_ctas - 1) / n_ctas;
-        const long cost = waves * tm;
-        if (best_cost < 0 || cost < best_cost) best_cost = cost, best = tm;
-    }
-    return best;
+void TileFamily::setup(int L, int n_sms) {
+    available = covers(L);
+    // consumer warpgroups (one active warp per 128 hidden columns) + one producer warpgroup (setmaxnreg split)
+    threads = ((L / 128 + 3) / 4) * 128 + 128;
+    smem = ((size_t)L * MP + MP * OUT_LD + MP * 4 + (size_t)NSTAGE * KC * L) * sizeof(float) + 2 * NSTAGE * sizeof(uint64_t) + 16;
+    int ctas_per_sm = (int)((227 * 1024) / (smem + 1024));
+    if (ctas_per_sm < 1) ctas_per_sm = 1;
+    if (ctas_per_sm > 4) ctas_per_sm = 4;
+    if (ctas_per_sm > 65536 / (threads * 168)) ctas_per_sm = 65536 / (threads * 168) > 0 ? 65536 / (threads * 168) : 1;
+    max_ctas[0] = n_sms * (ctas_per_sm > 2 ? 2 : ctas_per_sm);  // a residual in Tensor Memory allows 2 CTAs per SM
+    max_ctas[1] = n_sms * ctas_per_sm;
 }
 
 template <int TM>
@@ -884,363 +558,63 @@ static cudaError_t launch_fwd(const FwdParams& p, int grid, int threads, size_t 
     return cudaGetLastError();
 }
 
-extern "C" int mlb_forward(mlb_handle h, const mlb_forward_args* a, void* stream) {
-    if (!h || !a) return fail("mlb_forward: null argument");
-    if (a->n_rows < 0) return fail("mlb_forward: negative n_rows");
-    if (a->n_gather < 0 || a->n_gather > MLB_MAX_PEERS) return fail("mlb_forward: n_gather out of range");
-    const bool sync_gather = a->n_gather > 0 && a->gather_epoch != 0;
-    if (sync_gather) {
-        if (a->gather_rank < 0 || a->gather_rank >= a->n_gather) return fail("mlb_forward: gather_rank out of range");
-        for (int i = 0; i < a->n_gather; ++i)
-            if (!a->gather_flags[i]) return fail("mlb_forward: null gather_flags pointer");
-    }
-    if (a->n_rows == 0) {
-        if (!sync_gather) return 0;
-        // empty shard: this rank still publishes its epoch and waits for the others
-        CU(cudaSetDevice(h->device));
-        FwdParams pe;
-        memset(&pe, 0, sizeof(pe));
-        pe.n_gather = a->n_gather, pe.gather_epoch = a->gather_epoch, pe.gather_rank = a->gather_rank;
-        for (int i = 0; i < a->n_gather; ++i) pe.gather_flags[i] = a->gather_flags[i];
-        pe.err_flag = h->err_flag_dev;
-        pe.gather_done = h->gather_done;
-        pe.gather_done_target = ++h->gather_done_count;
-        gather_flag_only_kernel<<<1, 1, 0, (cudaStream_t)stream>>>(pe);
-        CU(cudaGetLastError());
-        g_launches++;
-        return 0;
-    }
-    if (!a->x || !a->out_raw) return fail("mlb_forward: x and out_raw are required");
-    const mlb_model_desc& d = h->desc;
-    if (a->input_kind == MLB_IN_KPS && d.input_size != 34) return fail("mlb_forward: MLB_IN_KPS needs a 34-d model");
-    if (a->input_kind == MLB_IN_KPS_STEREO) {
-        if (d.input_size != 68) return fail("mlb_forward: MLB_IN_KPS_STEREO needs a 68-d model");
-        if (!a->x_right || a->n_left < 1 || a->n_right < 1 || (long long)a->n_left * a->n_right != a->n_rows)
-            return fail("mlb_forward: stereo needs x_right and n_rows == n_left * n_right");
-    }
-    if (a->input_kind < MLB_IN_X || a->input_kind > MLB_IN_KPS_STEREO) return fail("mlb_forward: bad input_kind");
-    if ((a->flags & MLB_FWD_ZERO_CENTER) && a->input_kind != MLB_IN_KPS) return fail("mlb_forward: zero_center needs MLB_IN_KPS");
-    CU(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-
-    FwdParams p;
-    memset(&p, 0, sizeof(p));
-    p.blob = h->blob_dev;
-    memcpy(p.ops, h->ops, sizeof(mlb_op) * d.n_ops);
-    p.n_ops = d.n_ops;
-    p.in_size = d.input_size;
-    p.out_size = d.output_size;
-    p.L = d.linear_size;
-    p.decode_kind = d.decode_kind;
-    p.input_kind = a->input_kind;
-    p.flags = a->flags;
-    // residual stash: Tensor Memory by default (no DRAM write-back traffic, measured 0.5-5 % faster), scratch on request
-    if (a->flags & MLB_FWD_RES_SCRATCH) p.flags &= ~MLB_FWD_RES_TMEM; else p.flags |= MLB_FWD_RES_TMEM;
-    p.n_rows = a->n_rows;
-    p.n_right = a->n_right > 0 ? a->n_right : 1;
-    p.kpad0 = h->ops[0].Kpad;
-    memcpy(p.kinv, a->kinv, sizeof(p.kinv));
-    p.z_met = a->z_met != 0.f ? a->z_met : 10.f;
-    p.x = a->x;
-    p.xr = a->x_right;
-    p.out_raw = a->out_raw;
-    p.out_dec = a->out_dec;
-    p.out_xyzc = a->out_xyzc;
-    p.out_x = a->out_x;
-    p.drop_mask = a->drop_mask;
-    p.drop_seed = a->drop_seed;
-    p.p_drop = d.p_dropout;
-    p.res_scratch = h->res_scratch;
-    p.err_flag = h->err_flag_dev;
-    p.n_gather = a->n_gather;
-    p.gather_row0 = a->gather_row0;
-    for (int i = 0; i < a->n_gather; ++i) {
-        if (!a->gather[i]) return fail("mlb_forward: null gather pointer");
-        p.gather[i] = a->gather[i];
-        p.gather_flags[i] = sync_gather ? a->gather_flags[i] : nullptr;
-    }
-    p.gather_rank = a->gather_rank;
-    p.gather_done = h->gather_done;
-    p.gather_epoch = 0;  // set, together with the arrival target, on the launch that completes the batch
-    auto arm_gather = [&](unsigned arrivals) {
-        if (!sync_gather) return;
-        p.gather_epoch = a->gather_epoch;
-        h->gather_done_count += arrivals;
-        p.gather_done_target = h->gather_done_count;
-    };
-
-    // ---- large batches (and every batch of a model wider than the FFMA kernels cover): error-compensated TF32 on the
-    // tensor cores, persistent clusters over 128-row tiles (forward_tc.cu)
-    const bool forced_ffma = (a->flags & (MLB_FWD_FORCE_TILE | MLB_FWD_FORCE_CLUSTER | MLB_FWD_FORCE_WIDE)) != 0 || a->rows_per_group != 0;
-    if ((a->flags & MLB_FWD_FORCE_TC) && h->tc == nullptr)
-        return fail("mlb_forward: the tensor-core kernel is not available for this model (linear_size % 256 != 0)");
-    if (!h->ffma_ok && forced_ffma) return fail("mlb_forward: this model width runs on the tensor-core kernel only");
-    bool pick_tc = false;
-    if (h->tc != nullptr && !forced_ffma && h->ffma_ok && a->n_rows > 64) {
-        // measured wave times (calibrate()): tensor-core waves of 128-row tiles against the better of FFMA clusters / row tiles
-        const int tc_cl = mlb_tc_clusters(h->tc, 1 << 30);
-        const long tc_tiles = (a->n_rows + 127) / 128;
-        const double t_tc = h->t_tc_wave * (double)((tc_tiles + tc_cl - 1) / tc_cl);
-        double t_ffma = 1e30;
-        if (h->slab_dev != nullptr) t_ffma = h->t_cluster_wave * (double)(((a->n_rows + 15) / 16 + h->small_conc - 1) / h->small_conc);
-        const int tmc = pick_rows_per_group(a->n_rows, h->n_sms);
-        const long tl = (a->n_rows + 2 * tmc - 1) / (2 * tmc);
-        const double t_tl = (h->t_tile_a + h->t_tile_b * tmc) * (double)((tl + h->n_sms - 1) / h->n_sms);
-        if (t_tl < t_ffma) t_ffma = t_tl;
-        pick_tc = t_tc < t_ffma;
-        if (getenv("MLB_TC_MIN_ROWS")) pick_tc = a->n_rows >= h->tc_min_rows;
-    }
-    if (h->tc != nullptr && ((a->flags & MLB_FWD_FORCE_TC) || !h->ffma_ok || pick_tc)) {
-        p.flags &= ~MLB_FWD_RES_TMEM;
-        arm_gather((unsigned)mlb_tc_clusters(h->tc, a->n_rows));  // one arrival per cluster leader
-        cudaError_t et = mlb_tc_launch(h->tc, p, st);
-        if (et != cudaSuccess) return fail(std::string("loco_forward_tc_kernel launch: ") + cudaGetErrorString(et));
-        g_launches++;
-        h->last_kernel = MLB_KERNEL_TC;
-        return 0;
-    }
-
-    // ---- up to 16 detections (most images): the second-generation latency kernel (forward_wide2.cu): 2-D K x N split in
-    // 4-CTA clusters, partial sums through distributed shared memory, (value, epoch) exchange instead of barrier + copy
-    const bool forced_any = (a->flags & (MLB_FWD_FORCE_TILE | MLB_FWD_FORCE_CLUSTER | MLB_FWD_FORCE_WIDE | MLB_FWD_FORCE_TC)) != 0 ||
-                            a->rows_per_group != 0;
-    if ((a->flags & MLB_FWD_FORCE_WIDE2) && (h->w2slab_dev == nullptr || a->n_rows > 16))
-        return fail("mlb_forward: the second-generation latency kernel needs <= 16 rows and a supported model / device");
-    if (h->w2slab_dev != nullptr && a->n_rows <= 16 && ((a->flags & MLB_FWD_FORCE_WIDE2) || (!forced_any && !h->wide2_disabled))) {
-        p.n_tiles = 1, p.row_base = 0;
-        const unsigned done_before = h->gather_done_count;
-        arm_gather(1u);
-        const unsigned base = h->wide2_epoch;
-        cudaError_t ew = mlb_wide2_launch(p, h->w2slab_dev, h->w2slab_off, h->wide2_xg, h->wide2_hg, base, st);
-        if (ew == cudaSuccess) {
-            h->wide2_epoch = base + (unsigned)mlb_wide2_epochs(h->ops, d.n_ops);
-            g_launches++;
-            h->last_kernel = MLB_KERNEL_WIDE2;
-            return 0;
-        }
-        if (a->flags & MLB_FWD_FORCE_WIDE2) return fail(std::string("loco_forward_wide2_kernel launch: ") + cudaGetErrorString(ew));
-        cudaGetLastError();   // e.g. no cooperative launch under this context: use the other kernels from now on
-        h->wide2_disabled = true;
-        h->gather_done_count = done_before;
-        p.gather_epoch = 0;
-    }
-
-    // ---- one image's worth of detections: the whole grid on one 32-row tile at a time (forward_wide.cu).  Measured 45 /
-    // 60 us per 16- / 32-row tile against 177 us for a wave of clusters: ahead up to two tiles.
-    const bool forced_other = (a->flags & (MLB_FWD_FORCE_TILE | MLB_FWD_FORCE_CLUSTER)) != 0 || a->rows_per_group != 0;
-    if ((a->flags & MLB_FWD_FORCE_WIDE) && h->wslab_dev == nullptr)
-        return fail("mlb_forward: the whole-grid kernel is not available for this model / device");
-    if (h->wslab_dev != nullptr && ((a->flags & MLB_FWD_FORCE_WIDE) || (!forced_other && !h->wide_disabled && a->n_rows <= 64))) {
-        p.n_tiles = 1;
-        bool wide_ok = true;
-        for (int row0 = 0; row0 < a->n_rows; row0 += 32) {
-            p.row_base = row0;
-            const bool last_launch = row0 + 32 >= a->n_rows;
-            const unsigned done_before = h->gather_done_count;
-            if (last_launch) arm_gather(1u);
-            const unsigned base = h->wide_bar_count;
-            h->wide_bar_count += (unsigned)mlb_wide_barriers(h->ops, d.n_ops) * (unsigned)(d.linear_size / 8);
-            cudaError_t ew = mlb_wide_launch(p, h->wslab_dev, h->wslab_off, h->wide_xg, h->wide_bar, base, st);
-            if (ew != cudaSuccess) {
-                h->wide_bar_count = base;  // nothing ran: the device counters did not move
-                h->gather_done_count = done_before;
-                p.gather_epoch = 0;
-                if ((a->flags & MLB_FWD_FORCE_WIDE) || row0 > 0)
-                    return fail(std::string("loco_forward_wide_kernel launch: ") + cudaGetErrorString(ew));
-                // e.g. no cooperative launch under this context (MPS / partitioned SMs): use the other kernels from now on
-                cudaGetLastError();
-                wide_ok = false;
-                break;
-            }
-            g_launches++;
-        }
-        if (wide_ok) {
-            h->last_kernel = MLB_KERNEL_WIDE;
-            return 0;
-        }
-        h->wide_disabled = true;
-        p.row_base = 0;
-    }
-
-    // ---- small batches: 8-CTA cluster per 16 detections (forward_small.cu) when that finishes sooner than row tiles.
-    // Cost model, measured on this device at mlb_create (calibrate()): cluster wave for `small_conc` clusters; tile wave a + b TM.
-    if (h->slab_dev != nullptr && !(a->flags & MLB_FWD_FORCE_TILE)) {
-        const int n_clusters = (a->n_rows + 15) / 16;
-        const int conc = h->small_conc;
-        const double t_small = h->t_cluster_wave * ((n_clusters + conc - 1) / conc);
-        const int tm0 = pick_rows_per_group(a->n_rows, h->n_sms);
-        const long tiles0 = (a->n_rows + 2 * tm0 - 1) / (2 * tm0);
-        const double t_tile = (h->t_tile_a + h->t_tile_b * tm0) * ((tiles0 + h->n_sms - 1) / h->n_sms);
-        if ((a->flags & MLB_FWD_FORCE_CLUSTER) || (a->rows_per_group == 0 && t_small < t_tile)) {
-            p.n_tiles = n_clusters;
-            arm_gather((unsigned)(n_clusters < conc ? n_clusters : conc));  // one arrival per cluster leader
-            cudaError_t es = mlb_small_launch(p, h->slab_dev, h->slab_off, n_clusters < conc ? n_clusters : conc, st);
-            if (es != cudaSuccess) return fail(std::string("loco_forward_cluster_kernel launch: ") + cudaGetErrorString(es));
-            g_launches++;
-            h->last_kernel = MLB_KERNEL_CLUSTER;
-            return 0;
-        }
-    } else if (a->flags & MLB_FWD_FORCE_CLUSTER) {
-        return fail("mlb_forward: the cluster kernel needs linear_size == 1024");
-    }
-
-    // consumer warpgroups (one active warp per 128 hidden columns) + one producer warpgroup (setmaxnreg split)
-    const int threads = ((d.linear_size / 128 + 3) / 4) * 128 + 128;
-    const size_t smem = fwd_smem_bytes(d.linear_size);
-    int ctas_per_sm = (int)((227 * 1024) / (smem + 1024));
-    if (ctas_per_sm < 1) ctas_per_sm = 1;
-    if (ctas_per_sm > 4) ctas_per_sm = 4;
-    if (ctas_per_sm > 65536 / (threads * 168)) ctas_per_sm = 65536 / (threads * 168) > 0 ? 65536 / (threads * 168) : 1;
-    if (p.flags & MLB_FWD_RES_TMEM) ctas_per_sm = ctas_per_sm > 2 ? 2 : ctas_per_sm;
-    const int max_ctas = h->n_sms * ctas_per_sm;
-    int tm = a->rows_per_group;
-    if (tm == 0) tm = pick_rows_per_group(a->n_rows, max_ctas);
-    if (tm < 8 || tm > 16 || (tm & 1)) return fail("mlb_forward: rows_per_group must be 0 or one of 8,10,12,14,16");
-    p.n_tiles = (a->n_rows + 2 * tm - 1) / (2 * tm);
-    const int grid = p.n_tiles < max_ctas ? p.n_tiles : max_ctas;
-    if ((size_t)grid * 128 * 256 > h->res_floats) return fail("mlb_forward: residual scratch too small");
-
-    arm_gather((unsigned)grid);  // every CTA owns >= 1 tile and arrives once
+cudaError_t TileFamily::launch(FwdParams p, const FwdPlan& pl, cudaStream_t st, int* issued) const {
+    p.n_tiles = (p.n_rows + 2 * pl.tm - 1) / (2 * pl.tm);
     cudaError_t e;
-    switch (tm) {
-        case 8: e = launch_fwd<8>(p, grid, threads, smem, st); break;
-        case 10: e = launch_fwd<10>(p, grid, threads, smem, st); break;
-        case 12: e = launch_fwd<12>(p, grid, threads, smem, st); break;
-        case 14: e = launch_fwd<14>(p, grid, threads, smem, st); break;
-        default: e = launch_fwd<16>(p, grid, threads, smem, st); break;
+    switch (pl.tm) {
+        case 8: e = launch_fwd<8>(p, pl.grid, threads, smem, st); break;
+        case 10: e = launch_fwd<10>(p, pl.grid, threads, smem, st); break;
+        case 12: e = launch_fwd<12>(p, pl.grid, threads, smem, st); break;
+        case 14: e = launch_fwd<14>(p, pl.grid, threads, smem, st); break;
+        default: e = launch_fwd<16>(p, pl.grid, threads, smem, st); break;
     }
-    if (e != cudaSuccess) return fail(std::string("loco_forward_kernel launch: ") + cudaGetErrorString(e));
-    g_launches++;
-    h->last_kernel = MLB_KERNEL_TILE;
-    return 0;
-}
-
-static int ensure(float** buf, size_t floats) {
-    if (*buf) cudaFree(*buf);
-    *buf = nullptr;
-    CU(cudaMalloc(buf, floats * sizeof(float)));
-    return 0;
-}
-
-extern "C" int mlb_forward_host(mlb_handle h, const mlb_forward_args* a, void* stream) {
-    if (!h || !a) return fail("mlb_forward_host: null argument");
-    if (a->n_rows == 0) return 0;
-    if (!a->x || !a->out_raw) return fail("mlb_forward_host: x and out_raw are required");
-    CU(cudaSetDevice(h->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    const mlb_model_desc& d = h->desc;
-    const size_t B = (size_t)a->n_rows;
-    const bool stereo = a->input_kind == MLB_IN_KPS_STEREO;
-    const size_t in_rows = stereo ? (size_t)a->n_left : B;
-    const size_t in_w = a->input_kind == MLB_IN_X ? (size_t)d.input_size : 51;
-    if (B > h->st_rows || in_rows > h->st_rows) {
-        const size_t cap = B > in_rows ? B : in_rows;
-        if (ensure(&h->st_in, cap * 68)) return -1;
-        if (ensure(&h->st_raw, cap * OUT_LD)) return -1;
-        if (ensure(&h->st_dec, cap * 8)) return -1;
-        if (ensure(&h->st_xyzc, cap * 4)) return -1;
-        if (ensure(&h->st_x, cap * 68)) return -1;
-        h->st_rows = cap;
-    }
-    if (stereo && (size_t)a->n_right > h->st_rows_r) {
-        if (ensure(&h->st_in_r, (size_t)a->n_right * 51)) return -1;
-        h->st_rows_r = (size_t)a->n_right;
-    }
-    CU(cudaMemcpyAsync(h->st_in, a->x, in_rows * in_w * sizeof(float), cudaMemcpyHostToDevice, st));
-    if (stereo) {
-        if (!a->x_right) return fail("mlb_forward_host: stereo needs x_right");
-        CU(cudaMemcpyAsync(h->st_in_r, a->x_right, (size_t)a->n_right * 51 * sizeof(float), cudaMemcpyHostToDevice, st));
-    }
-    mlb_forward_args dev = *a;
-    dev.x = h->st_in;
-    dev.x_right = stereo ? h->st_in_r : nullptr;
-    dev.out_raw = h->st_raw;
-    dev.out_dec = a->out_dec ? h->st_dec : nullptr;
-    dev.out_xyzc = a->out_xyzc ? h->st_xyzc : nullptr;
-    dev.out_x = a->out_x ? h->st_x : nullptr;
-    dev.drop_mask = nullptr;
-    dev.n_gather = 0;
-    if (a->drop_mask) return fail("mlb_forward_host: drop_mask is a device-only option");
-    // One image's worth of rows: the kernel stores straight into the caller's buffers when they are pinned (mapped under
-    // UVA) -- a few posted PCIe writes from one CTA instead of three D2H copies.  Larger batches keep the DMA copies
-    // (row-at-a-time stores would turn into ~12 small PCIe writes per detection).
-    bool zero_copy = B <= 64;
-    void* dptr[4] = {nullptr, nullptr, nullptr, nullptr};
-    if (zero_copy) {
-        void* hp[4] = {a->out_raw, a->out_dec, a->out_xyzc, a->out_x};
-        for (int i = 0; i < 4 && zero_copy; ++i) {
-            if (!hp[i]) continue;
-            cudaPointerAttributes at;
-            if (cudaPointerGetAttributes(&at, hp[i]) != cudaSuccess || at.type != cudaMemoryTypeHost || !at.devicePointer) {
-                cudaGetLastError();
-                zero_copy = false;
-            } else {
-                dptr[i] = at.devicePointer;
-            }
-        }
-    }
-    if (zero_copy) {
-        dev.out_raw = static_cast<float*>(dptr[0]);
-        dev.out_dec = static_cast<float*>(dptr[1]);
-        dev.out_xyzc = static_cast<float*>(dptr[2]);
-        dev.out_x = static_cast<float*>(dptr[3]);
-    }
-    if (mlb_forward(h, &dev, stream)) return -1;
-    if (!zero_copy) {
-        CU(cudaMemcpyAsync(a->out_raw, h->st_raw, B * d.output_size * sizeof(float), cudaMemcpyDeviceToHost, st));
-        if (a->out_dec) CU(cudaMemcpyAsync(a->out_dec, h->st_dec, B * 8 * sizeof(float), cudaMemcpyDeviceToHost, st));
-        if (a->out_xyzc) CU(cudaMemcpyAsync(a->out_xyzc, h->st_xyzc, B * 4 * sizeof(float), cudaMemcpyDeviceToHost, st));
-        if (a->out_x) CU(cudaMemcpyAsync(a->out_x, h->st_x, B * d.input_size * sizeof(float), cudaMemcpyDeviceToHost, st));
-    }
-    CU(cudaStreamSynchronize(st));
-    const int err = *reinterpret_cast<volatile int*>(h->err_flag_host);
-    if (err) return fail("mlb_forward_host: device error flag " + std::to_string(err));
-    return 0;
+    if (e == cudaSuccess) ++*issued;
+    return e;
 }
 
 extern "C" int mlb_preprocess(const float* kps, int n_rows, const float kinv[9], float z_met, int zero_center, float* out_x,
                               void* stream) {
     if (n_rows == 0) return 0;
-    if (!kps || !kinv || !out_x || n_rows < 0) return fail("mlb_preprocess: bad argument");
+    if (!kps || !kinv || !out_x || n_rows < 0) return mlb_fail("mlb_preprocess: bad argument");
     const int wpb = 8;
     preprocess_kernel<<<(n_rows + wpb - 1) / wpb, wpb * 32, 0, (cudaStream_t)stream>>>(
         kps, n_rows, kinv[0], kinv[1], kinv[2], kinv[3], kinv[4], kinv[5], z_met != 0.f ? z_met : 10.f, zero_center, out_x);
-    CU(cudaGetLastError());
-    g_launches++;
+    MLB_CU(cudaGetLastError());
+    mlb_count_launch();
     return 0;
 }
 
 extern "C" int mlb_decode(const float* raw, int n_rows, int out_size, int decode_kind, float* dec, void* stream) {
     if (n_rows == 0) return 0;
-    if (!raw || !dec || n_rows < 0 || out_size < 1 || out_size > OUT_LD) return fail("mlb_decode: bad argument");
-    if (decode_kind == MLB_DECODE_LOCO && out_size < 9) return fail("mlb_decode: extract_outputs needs >= 9 columns");
-    if (decode_kind == MLB_DECODE_MONO && out_size < 9) return fail("mlb_decode: extract_outputs_mono needs 9 columns");
-    if (decode_kind == MLB_DECODE_DB && out_size < 2) return fail("mlb_decode: needs 2 columns");
+    if (!raw || !dec || n_rows < 0 || out_size < 1 || out_size > OUT_LD) return mlb_fail("mlb_decode: bad argument");
+    if (decode_kind == MLB_DECODE_LOCO && out_size < 9) return mlb_fail("mlb_decode: extract_outputs needs >= 9 columns");
+    if (decode_kind == MLB_DECODE_MONO && out_size < 9) return mlb_fail("mlb_decode: extract_outputs_mono needs 9 columns");
+    if (decode_kind == MLB_DECODE_DB && out_size < 2) return mlb_fail("mlb_decode: needs 2 columns");
     decode_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(raw, n_rows, out_size, decode_kind, dec);
-    CU(cudaGetLastError());
-    g_launches++;
+    MLB_CU(cudaGetLastError());
+    mlb_count_launch();
     return 0;
 }
 
 extern "C" int mlb_laplace_std(const float* d_bi, int n_pass, int n_rows, int n_samples, uint64_t seed, float* out_std,
                                void* stream) {
     if (n_rows == 0) return 0;
-    if (!d_bi || !out_std || n_pass < 1 || n_rows < 0 || n_samples < 1) return fail("mlb_laplace_std: bad argument");
+    if (!d_bi || !out_std || n_pass < 1 || n_rows < 0 || n_samples < 1) return mlb_fail("mlb_laplace_std: bad argument");
     laplace_std_kernel<<<(n_rows + 127) / 128, 128, 0, (cudaStream_t)stream>>>(d_bi, n_pass, n_rows, n_samples, seed, out_std);
-    CU(cudaGetLastError());
-    g_launches++;
+    MLB_CU(cudaGetLastError());
+    mlb_count_launch();
     return 0;
 }
 
 extern "C" int mlb_ipc_alloc(int device, size_t bytes, void** dev_ptr, unsigned char handle[MLB_IPC_HANDLE_BYTES]) {
-    if (!dev_ptr || !handle || bytes == 0) return fail("mlb_ipc_alloc: bad argument");
+    if (!dev_ptr || !handle || bytes == 0) return mlb_fail("mlb_ipc_alloc: bad argument");
     static_assert(sizeof(cudaIpcMemHandle_t) <= MLB_IPC_HANDLE_BYTES, "handle size");
-    CU(cudaSetDevice(device));
+    MLB_CU(cudaSetDevice(device));
     void* ptr = nullptr;
-    CU(cudaMalloc(&ptr, bytes));
-    CU(cudaMemset(ptr, 0, bytes));
+    MLB_CU(cudaMalloc(&ptr, bytes));
+    MLB_CU(cudaMemset(ptr, 0, bytes));
     cudaIpcMemHandle_t hd;
-    CU(cudaIpcGetMemHandle(&hd, ptr));
+    MLB_CU(cudaIpcGetMemHandle(&hd, ptr));
     memset(handle, 0, MLB_IPC_HANDLE_BYTES);
     memcpy(handle, &hd, sizeof(hd));
     *dev_ptr = ptr;
@@ -1248,37 +622,37 @@ extern "C" int mlb_ipc_alloc(int device, size_t bytes, void** dev_ptr, unsigned 
 }
 
 extern "C" int mlb_ipc_open(int device, const unsigned char handle[MLB_IPC_HANDLE_BYTES], void** dev_ptr) {
-    if (!dev_ptr || !handle) return fail("mlb_ipc_open: bad argument");
-    CU(cudaSetDevice(device));
+    if (!dev_ptr || !handle) return mlb_fail("mlb_ipc_open: bad argument");
+    MLB_CU(cudaSetDevice(device));
     cudaIpcMemHandle_t hd;
     memcpy(&hd, handle, sizeof(hd));
     void* ptr = nullptr;
-    CU(cudaIpcOpenMemHandle(&ptr, hd, cudaIpcMemLazyEnablePeerAccess));
+    MLB_CU(cudaIpcOpenMemHandle(&ptr, hd, cudaIpcMemLazyEnablePeerAccess));
     *dev_ptr = ptr;
     return 0;
 }
 
 extern "C" int mlb_ipc_close(void* dev_ptr) {
-    if (dev_ptr) CU(cudaIpcCloseMemHandle(dev_ptr));
+    if (dev_ptr) MLB_CU(cudaIpcCloseMemHandle(dev_ptr));
     return 0;
 }
 
 extern "C" int mlb_ipc_free(void* dev_ptr) {
-    if (dev_ptr) CU(cudaFree(dev_ptr));
+    if (dev_ptr) MLB_CU(cudaFree(dev_ptr));
     return 0;
 }
 
 extern "C" int mlb_probe_ffma(int device, int blocks, int iters, double* flops, void* stream) {
-    CU(cudaSetDevice(device));
+    MLB_CU(cudaSetDevice(device));
     static float* sink = nullptr;
-    if (!sink) CU(cudaMalloc(&sink, 16));
+    if (!sink) MLB_CU(cudaMalloc(&sink, 16));
     if (iters < 0)
         ffma2_probe_kernel<<<blocks, 512, 0, (cudaStream_t)stream>>>(-iters, sink);  // packed fma.rn.f32x2 variant
     else
         ffma_probe_kernel<<<blocks, 512, 0, (cudaStream_t)stream>>>(iters, sink);
-    CU(cudaGetLastError());
+    MLB_CU(cudaGetLastError());
     if (iters < 0) iters = -iters;
-    g_launches++;
+    mlb_count_launch();
     if (flops) *flops = (double)blocks * 512.0 * (double)iters * 8.0 * 16.0 * 2.0;
     return 0;
 }

@@ -13,9 +13,7 @@
 #include <stdint.h>
 #include <string.h>
 
-#include <string>
-
-#include "fwd_common.cuh"
+#include "fwd_family.cuh"
 
 namespace mlb {
 
@@ -356,26 +354,21 @@ __global__ void slab_pack_kernel(const float* __restrict__ wt, float* __restrict
 
 using namespace mlb;
 
-size_t mlb_small_smem_bytes(int L) {
+static size_t small_smem_bytes(int L) {
     const size_t fl = (size_t)L * SR + 8 * SR * SC + 8 * SNST * SCHUNK + SR * OUT_LD + SR * 4;
     return fl * sizeof(float) + 8 * SNST * sizeof(uint64_t) + 16;
 }
 
-cudaError_t mlb_small_pack(const float* blob, const mlb_op* ops, int n_ops, int L, float* slab, long long* slab_off,
-                           cudaStream_t st) {
-    long long off = 0;
-    for (int i = 0; i < n_ops; ++i) {
-        slab_off[i] = off;
-        if (ops[i].type != MLB_OP_GEMM) continue;
-        slab_pack_kernel<<<256, 256, 0, st>>>(blob + ops[i].w_off, slab + off, ops[i].Kpad, L);
-        off += (long long)ops[i].Kpad * L;
-    }
+cudaError_t ClusterFamily::repack(const float* blob, const mlb_op* ops, int n_ops, int L, cudaStream_t st) const {
+    if (!available) return cudaSuccess;
+    for (int i = 0; i < n_ops; ++i)
+        if (ops[i].type == MLB_OP_GEMM) slab_pack_kernel<<<256, 256, 0, st>>>(blob + ops[i].w_off, slab + slab_off[i], ops[i].Kpad, L);
     return cudaGetLastError();
 }
 
 // how many 8-CTA clusters of this kernel can be resident at once (GPC packing decides: measured 11-16 on a B200)
-int mlb_small_max_clusters(int L) {
-    const size_t smem = mlb_small_smem_bytes(L);
+static int small_max_clusters(int L) {
+    const size_t smem = small_smem_bytes(L);
     if (cudaFuncSetAttribute(loco_forward_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) return 0;
     cudaLaunchConfig_t cfg;
     memset(&cfg, 0, sizeof(cfg));
@@ -395,13 +388,37 @@ int mlb_small_max_clusters(int L) {
     return n;
 }
 
-cudaError_t mlb_small_launch(const FwdParams& p, const float* slab, const long long* slab_off, int n_clusters, cudaStream_t st) {
+cudaError_t ClusterFamily::setup(const float* blob, const mlb_op* ops, int n_ops, int L) {
+    if (L != 1024) return cudaSuccess;
+    long long off = 0;
+    for (int i = 0; i < n_ops; ++i) {
+        slab_off[i] = off;
+        if (ops[i].type == MLB_OP_GEMM) off += (long long)ops[i].Kpad * L;
+    }
+    cudaError_t e = cudaMalloc(&slab, (size_t)off * sizeof(float));
+    if (e != cudaSuccess) return e;
+    available = true;
+    if ((e = repack(blob, ops, n_ops, L, 0)) != cudaSuccess) return e;
+    conc = small_max_clusters(L);
+    if (conc < 1) conc = 8;
+    return cudaSuccess;
+}
+
+void ClusterFamily::release() {
+    cudaFree(slab);
+    slab = nullptr;
+    available = false;
+}
+
+cudaError_t ClusterFamily::launch(FwdParams p, const FwdPlan& pl, cudaStream_t st, int* issued) const {
     SmallExtra ex;
     ex.slab = slab;
     memcpy(ex.slab_off, slab_off, sizeof(ex.slab_off));
-    const size_t smem = mlb_small_smem_bytes(p.L);
+    p.n_tiles = (p.n_rows + 15) / 16;
+    const size_t smem = small_smem_bytes(p.L);
     cudaError_t e = cudaFuncSetAttribute(loco_forward_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    loco_forward_cluster_kernel<<<n_clusters * CL, 256, smem, st>>>(p, ex);
-    return cudaGetLastError();
+    loco_forward_cluster_kernel<<<pl.clusters * CL, 256, smem, st>>>(p, ex);
+    if ((e = cudaGetLastError()) == cudaSuccess) ++*issued;
+    return e;
 }

@@ -26,12 +26,9 @@
 //                the bbox-centre ray, fused all-gather peers), exactly the epilogue of the FFMA kernels (fwd_common.cuh).
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <stdlib.h>
 #include <string.h>
 
-#include <string>
-
-#include "fwd_common.cuh"
+#include "fwd_family.cuh"
 
 namespace mlb {
 
@@ -595,19 +592,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) loco_forward_tc_kernel(const __
 // ================================================================================================ host side
 using namespace mlb;
 
-cudaError_t mlb_tc_set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_tc_marks, &ptr, sizeof(ptr)); }
-
-struct mlb_tc_state {
-    float* wplanes[MLB_MAX_OPS];
-    int n_kb[MLB_MAX_OPS];
-    float* ws;
-    size_t slot_floats;
-    int max_clusters;
-    int nct;     // CTAs per cluster = L / 256
-};
-
-// widths the tensor-core kernel covers: 256 output columns per CTA, clusters of up to 8 CTAs
-bool mlb_tc_supported(int L) { return L >= TCN && L % TCN == 0 && L / TCN <= TC_MAX_CT; }
+cudaError_t TcFamily::set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_tc_marks, &ptr, sizeof(ptr)); }
 
 static void tc_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at, int clusters, int nct, cudaStream_t st) {
     memset(cfg, 0, sizeof(*cfg));
@@ -621,65 +606,61 @@ static void tc_config(cudaLaunchConfig_t* cfg, cudaLaunchAttribute* at, int clus
     cfg->numAttrs = 1;
 }
 
-// pack the weight planes, size the workspace (one slot per co-resident cluster).  Returns nullptr + *err on failure.
-mlb_tc_state* mlb_tc_prepare(const float* blob_dev, const mlb_op* ops, int n_ops, int L, cudaStream_t st, cudaError_t* err) {
-    mlb_tc_state* t = new mlb_tc_state();
-    memset(t, 0, sizeof(*t));
-    t->nct = L / TCN;
-    *err = cudaFuncSetAttribute(loco_forward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES);
-    if (*err != cudaSuccess) { delete t; return nullptr; }
-    int first = -1;
-    for (int i = 0; i < n_ops; ++i) {
-        if (ops[i].type != MLB_OP_GEMM) continue;
-        if (first < 0) first = i;
-        t->n_kb[i] = (ops[i].Kpad + TCKB - 1) / TCKB;
-        const size_t fl = (size_t)2 * t->n_kb[i] * TCKB * L;
-        if ((*err = cudaMalloc(&t->wplanes[i], fl * sizeof(float))) != cudaSuccess) return nullptr;
-        tc_pack_weights_kernel<<<296, 256, 0, st>>>(blob_dev + ops[i].w_off, t->wplanes[i], ops[i].Kpad, L, t->n_kb[i]);
-    }
-    cudaLaunchConfig_t cfg;
-    cudaLaunchAttribute at;
-    tc_config(&cfg, &at, 64, t->nct, st);
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, loco_forward_tc_kernel, &cfg) != cudaSuccess || n < 1) {
-        cudaGetLastError();
-        n = 148 / t->nct / 2;
-    }
-    if (getenv("MLB_TC_CLUSTERS") && atoi(getenv("MLB_TC_CLUSTERS")) > 0 && atoi(getenv("MLB_TC_CLUSTERS")) < n) n = atoi(getenv("MLB_TC_CLUSTERS"));
-    t->max_clusters = n;
-    const size_t plane = (size_t)TCM * TCKB;
-    t->slot_floats = (size_t)t->n_kb[first] * 2 * plane + 2 * (size_t)(L / TCKB) * 2 * plane + (size_t)TCM * L;
-    if ((*err = cudaMalloc(&t->ws, (size_t)n * t->slot_floats * sizeof(float))) != cudaSuccess) return nullptr;
-    if ((*err = cudaMemsetAsync(t->ws, 0, (size_t)n * t->slot_floats * sizeof(float), st)) != cudaSuccess) return nullptr;
-    *err = cudaGetLastError();
-    return t;
-}
-
-cudaError_t mlb_tc_repack(mlb_tc_state* t, const float* blob_dev, const mlb_op* ops, int n_ops, int L, cudaStream_t st) {
+cudaError_t TcFamily::repack(const float* blob, const mlb_op* ops, int n_ops, int L, cudaStream_t st) const {
+    if (!available) return cudaSuccess;
     for (int i = 0; i < n_ops; ++i)
         if (ops[i].type == MLB_OP_GEMM)
-            tc_pack_weights_kernel<<<296, 256, 0, st>>>(blob_dev + ops[i].w_off, t->wplanes[i], ops[i].Kpad, L, t->n_kb[i]);
+            tc_pack_weights_kernel<<<296, 256, 0, st>>>(blob + ops[i].w_off, wplanes[i], ops[i].Kpad, L, n_kb[i]);
     return cudaGetLastError();
 }
 
-void mlb_tc_free(mlb_tc_state* t) {
-    if (!t) return;
-    for (int i = 0; i < MLB_MAX_OPS; ++i) cudaFree(t->wplanes[i]);
-    cudaFree(t->ws);
-    delete t;
+// widths the tensor-core kernel covers: 256 output columns per CTA, clusters of up to 8 CTAs
+bool TcFamily::covers(int L) { return L >= TCN && L % TCN == 0 && L / TCN <= TC_MAX_CT; }
+
+// pack the weight planes, size the workspace (one slot per co-resident cluster)
+cudaError_t TcFamily::setup(const float* blob, const mlb_op* ops, int n_ops, int L) {
+    if (!covers(L)) return cudaSuccess;
+    nct = L / TCN;
+    cudaError_t e = cudaFuncSetAttribute(loco_forward_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TC_SMEM_BYTES);
+    int first = -1;
+    for (int i = 0; i < n_ops && e == cudaSuccess; ++i) {
+        if (ops[i].type != MLB_OP_GEMM) continue;
+        if (first < 0) first = i;
+        n_kb[i] = (ops[i].Kpad + TCKB - 1) / TCKB;
+        e = cudaMalloc(&wplanes[i], (size_t)2 * n_kb[i] * TCKB * L * sizeof(float));
+    }
+    available = e == cudaSuccess;
+    if (e == cudaSuccess) e = repack(blob, ops, n_ops, L, 0);
+    if (e == cudaSuccess) {
+        cudaLaunchConfig_t cfg;
+        cudaLaunchAttribute at;
+        tc_config(&cfg, &at, 64, nct, 0);
+        if (cudaOccupancyMaxActiveClusters(&max_clusters, loco_forward_tc_kernel, &cfg) != cudaSuccess || max_clusters < 1) {
+            cudaGetLastError();
+            max_clusters = 148 / nct / 2;
+        }
+        const size_t plane = (size_t)TCM * TCKB;
+        slot_floats = (size_t)n_kb[first] * 2 * plane + 2 * (size_t)(L / TCKB) * 2 * plane + (size_t)TCM * L;
+        e = cudaMalloc(&ws, (size_t)max_clusters * slot_floats * sizeof(float));
+    }
+    if (e == cudaSuccess) e = cudaMemsetAsync(ws, 0, (size_t)max_clusters * slot_floats * sizeof(float), 0);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) release();
+    return e;
 }
 
-int mlb_tc_clusters(const mlb_tc_state* t, int n_rows) {
-    const int tiles = (n_rows + TCM - 1) / TCM;
-    return tiles < t->max_clusters ? tiles : t->max_clusters;
+void TcFamily::release() {
+    for (int i = 0; i < MLB_MAX_OPS; ++i) cudaFree(wplanes[i]), wplanes[i] = nullptr;
+    cudaFree(ws);
+    ws = nullptr;
+    available = false;
 }
-int mlb_tc_max_clusters(const mlb_tc_state* t) { return t->max_clusters; }
 
-cudaError_t mlb_tc_launch(const mlb_tc_state* t, const FwdParams& p, cudaStream_t st) {
+cudaError_t TcFamily::launch(FwdParams p, const FwdPlan& pl, cudaStream_t st, int* issued) const {
     TcExtra ex;
     memset(&ex, 0, sizeof(ex));
-    for (int i = 0; i < MLB_MAX_OPS; ++i) ex.wplanes[i] = t->wplanes[i], ex.n_kb[i] = t->n_kb[i];
-    ex.ws = t->ws, ex.slot_floats = t->slot_floats;
+    for (int i = 0; i < MLB_MAX_OPS; ++i) ex.wplanes[i] = wplanes[i], ex.n_kb[i] = n_kb[i];
+    ex.ws = ws, ex.slot_floats = slot_floats;
     ex.n_tiles = (p.n_rows + TCM - 1) / TCM;
     int last_gemm = -1;
     for (int i = 0; i < p.n_ops; ++i) {
@@ -696,8 +677,11 @@ cudaError_t mlb_tc_launch(const mlb_tc_state* t, const FwdParams& p, cudaStream_
             }
         }
     }
+    p.flags &= ~MLB_FWD_RES_TMEM;  // the residual always goes through the scratch here
     cudaLaunchConfig_t cfg;
     cudaLaunchAttribute at;
-    tc_config(&cfg, &at, mlb_tc_clusters(t, p.n_rows), t->nct, st);
-    return cudaLaunchKernelEx(&cfg, loco_forward_tc_kernel, p, ex);
+    tc_config(&cfg, &at, pl.clusters, nct, st);
+    cudaError_t e = cudaLaunchKernelEx(&cfg, loco_forward_tc_kernel, p, ex);
+    if (e == cudaSuccess) ++*issued;
+    return e;
 }

@@ -19,9 +19,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <string>
-
-#include "fwd_common.cuh"
+#include "fwd_family.cuh"
 
 namespace mlb {
 
@@ -262,7 +260,7 @@ static size_t wide_smem(int L) {
 
 using namespace mlb;
 
-cudaError_t mlb_wide_set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_wide_marks, &ptr, sizeof(ptr)); }
+cudaError_t WideFamily::set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_wide_marks, &ptr, sizeof(ptr)); }
 
 // head weights W[N][K] -> ceil(N/8) zero-padded k-major slabs [K][8]
 __global__ void wide_pack_head_kernel(const float* __restrict__ w, float* __restrict__ slab, int N, int K) {
@@ -275,21 +273,8 @@ __global__ void wide_pack_head_kernel(const float* __restrict__ w, float* __rest
     }
 }
 
-// total floats of the slab copy and each op's offset in it (GEMM: [L/8][Kpad][8]; head: [ceil(N/8)][K][8])
-size_t mlb_wide_slab_floats(const mlb_op* ops, int n_ops, int L, long long* slab_off) {
-    size_t off = 0;
-    for (int i = 0; i < n_ops; ++i) {
-        slab_off[i] = (long long)off;
-        if (ops[i].type == MLB_OP_GEMM)
-            off += (size_t)ops[i].Kpad * L;
-        else
-            off += (size_t)((ops[i].N + WC - 1) / WC) * ops[i].K * WC;
-    }
-    return off;
-}
-
-cudaError_t mlb_wide_pack(const float* blob, const mlb_op* ops, int n_ops, int L, float* slab, const long long* slab_off,
-                          cudaStream_t st) {
+cudaError_t WideFamily::repack(const float* blob, const mlb_op* ops, int n_ops, int L, cudaStream_t st) const {
+    if (!available) return cudaSuccess;
     for (int i = 0; i < n_ops; ++i) {
         if (ops[i].type == MLB_OP_GEMM)
             wide_pack_kernel<<<128, 256, 0, st>>>(blob + ops[i].w_off, slab + slab_off[i], ops[i].Kpad, L);
@@ -300,7 +285,7 @@ cudaError_t mlb_wide_pack(const float* blob, const mlb_op* ops, int n_ops, int L
 }
 
 // can the whole grid (L/8 CTAs) be co-resident?  (cooperative launch requirement)
-bool mlb_wide_supported(int L, int n_sms) {
+static bool wide_supported(int L, int n_sms) {
     if (L % 128 != 0 || L / WC > n_sms) return false;
     int occ = 0;
     if (cudaFuncSetAttribute(loco_forward_wide_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem<32>(L)) != cudaSuccess)
@@ -312,28 +297,57 @@ bool mlb_wide_supported(int L, int n_sms) {
     return true;
 }
 
-// number of grid barriers one launch performs (the host advances its copy of the counter by n * grid)
-int mlb_wide_barriers(const mlb_op* ops, int n_ops) {
-    int n = 0;
-    for (int i = 0; i < n_ops; ++i) n += ops[i].type == MLB_OP_GEMM;
-    return n;
+cudaError_t WideFamily::setup(const float* blob, const mlb_op* ops, int n_ops, int L, int n_sms) {
+    if (L > 1024 || !wide_supported(L, n_sms)) return cudaSuccess;
+    // slab copy: GEMM [L/8][Kpad][8]; head [ceil(N/8)][K][8]
+    size_t off = 0;
+    for (int i = 0; i < n_ops; ++i) {
+        slab_off[i] = (long long)off;
+        if (ops[i].type == MLB_OP_GEMM)
+            off += (size_t)ops[i].Kpad * L;
+        else
+            off += (size_t)((ops[i].N + WC - 1) / WC) * ops[i].K * WC;
+    }
+    cudaError_t e;
+    if ((e = cudaMalloc(&slab, off * sizeof(float))) != cudaSuccess) return e;
+    available = true;
+    if ((e = repack(blob, ops, n_ops, L, 0)) != cudaSuccess) return e;
+    if ((e = mlb_zalloc(&xg, (size_t)2 * L * 32 * sizeof(float))) != cudaSuccess) return e;
+    return mlb_zalloc(&bar, sizeof(unsigned));
 }
 
-cudaError_t mlb_wide_launch(const FwdParams& p, const float* wslab, const long long* wslab_off, float* xg, unsigned* bar,
-                            unsigned bar_base, cudaStream_t st) {
-    WideExtra ex;
-    ex.wslab = wslab;
-    for (int i = 0; i < MLB_MAX_OPS; ++i) ex.wslab_off[i] = i < p.n_ops ? wslab_off[i] : 0;
-    ex.xg = xg, ex.bar = bar, ex.bar_base = bar_base;
-    void* args[] = {(void*)&p, (void*)&ex};
-    const int grid = p.L / WC;
+void WideFamily::release() {
+    cudaFree(slab), cudaFree(xg), cudaFree(bar);
+    slab = nullptr, xg = nullptr, bar = nullptr;
+    available = false;
+}
+
+template <int R>
+static cudaError_t launch_wide(void** args, int L, cudaStream_t st) {
     // (the opt-in shared-memory size is a per-function, per-process attribute: set it for THIS model's width on every launch)
-    if (p.n_rows - p.row_base <= 16) {
-        cudaError_t e = cudaFuncSetAttribute(loco_forward_wide_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem<16>(p.L));
-        if (e != cudaSuccess) return e;
-        return cudaLaunchCooperativeKernel((void*)loco_forward_wide_kernel<16>, dim3(grid), dim3(WNT), args, wide_smem<16>(p.L), st);
-    }
-    cudaError_t e = cudaFuncSetAttribute(loco_forward_wide_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem<32>(p.L));
+    const cudaError_t e = cudaFuncSetAttribute(loco_forward_wide_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide_smem<R>(L));
     if (e != cudaSuccess) return e;
-    return cudaLaunchCooperativeKernel((void*)loco_forward_wide_kernel<32>, dim3(grid), dim3(WNT), args, wide_smem<32>(p.L), st);
+    return cudaLaunchCooperativeKernel((void*)loco_forward_wide_kernel<R>, dim3(L / WC), dim3(WNT), args, wide_smem<R>(L), st);
+}
+
+cudaError_t WideFamily::launch(FwdParams p, const FwdPlan& pl, cudaStream_t st, int* issued) {
+    WideExtra ex;
+    ex.wslab = slab;
+    for (int i = 0; i < MLB_MAX_OPS; ++i) ex.wslab_off[i] = i < p.n_ops ? slab_off[i] : 0;
+    ex.xg = xg, ex.bar = bar;
+    int n_gemm = 0;  // one grid barrier per GEMM: the counter advances by n_gemm * grid per launch
+    for (int i = 0; i < p.n_ops; ++i) n_gemm += p.ops[i].type == MLB_OP_GEMM;
+    const unsigned epoch = p.gather_epoch;
+    void* args[] = {(void*)&p, (void*)&ex};
+    p.n_tiles = 1;
+    for (int t = 0; t < pl.launches; ++t) {
+        p.row_base = 32 * t;
+        p.gather_epoch = t + 1 == pl.launches ? epoch : 0;  // the last launch completes the batch for the all-gather
+        ex.bar_base = bar_count;
+        const cudaError_t e = p.n_rows - p.row_base <= 16 ? launch_wide<16>(args, p.L, st) : launch_wide<32>(args, p.L, st);
+        if (e != cudaSuccess) return e;  // nothing ran: the device counter did not move
+        bar_count += (unsigned)n_gemm * (unsigned)(p.L / WC);
+        ++*issued;
+    }
+    return cudaSuccess;
 }

@@ -26,9 +26,7 @@
 #include <stdint.h>
 #include <string.h>
 
-#include <string>
-
-#include "fwd_common.cuh"
+#include "fwd_family.cuh"
 
 namespace mlb {
 
@@ -406,26 +404,17 @@ static size_t wide2_smem(int L) {
 
 using namespace mlb;
 
-cudaError_t mlb_wide2_set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_wide2_marks, &ptr, sizeof(ptr)); }
+cudaError_t Wide2Family::set_marks(unsigned long long* ptr) { return cudaMemcpyToSymbol(mlb::g_wide2_marks, &ptr, sizeof(ptr)); }
 
-size_t mlb_wide2_slab_floats(const mlb_op* ops, int n_ops, int L, long long* slab_off) {
-    size_t off = 0;
-    const int KS = L / W2_CL;
-    for (int i = 0; i < n_ops; ++i) {
-        slab_off[i] = (long long)off;
-        if (ops[i].type == MLB_OP_GEMM) off += (size_t)(L / W2_NC) * W2_CL * (ops[i].Kpad < KS ? ops[i].Kpad : KS) * W2_NC;
-    }
-    return off;
-}
-
-cudaError_t mlb_wide2_pack(const float* blob, const mlb_op* ops, int n_ops, int L, float* slab, const long long* slab_off, cudaStream_t st) {
+cudaError_t Wide2Family::repack(const float* blob, const mlb_op* ops, int n_ops, int L, cudaStream_t st) const {
+    if (!available) return cudaSuccess;
     for (int i = 0; i < n_ops; ++i)
         if (ops[i].type == MLB_OP_GEMM) wide2_pack_kernel<<<128, 256, 0, st>>>(blob + ops[i].w_off, slab + slab_off[i], ops[i].Kpad, L);
     return cudaGetLastError();
 }
 
 // all L/8 CTAs (L/32 clusters of 4) must be co-resident; heads and layer widths the kernel is written for
-bool mlb_wide2_supported(const mlb_op* ops, int n_ops, int L, int out_size, int n_sms) {
+static bool wide2_supported(const mlb_op* ops, int n_ops, int L, int out_size, int n_sms) {
     if (L % 128 != 0 || L / W2_FC > n_sms || out_size > W2_HQ) return false;
     for (int i = 0; i < n_ops; ++i)
         if (ops[i].type == MLB_OP_GEMM && (ops[i].flags & MLB_F_IN_XIN) && ops[i].Kpad > L / W2_CL) return false;
@@ -444,21 +433,34 @@ bool mlb_wide2_supported(const mlb_op* ops, int n_ops, int L, int out_size, int 
     return true;
 }
 
-int mlb_wide2_epochs(const mlb_op* ops, int n_ops) {   // epochs one launch consumes
-    int n = 0;
-    for (int i = 0; i < n_ops; ++i) n += ops[i].type == MLB_OP_GEMM;
-    return n + 2;
+cudaError_t Wide2Family::setup(const float* blob, const mlb_op* ops, int n_ops, int L, int out_size, int n_sms) {
+    if (L > 1024 || !wide2_supported(ops, n_ops, L, out_size, n_sms)) return cudaSuccess;
+    size_t off = 0;
+    const int KS = L / W2_CL;
+    for (int i = 0; i < n_ops; ++i) {
+        slab_off[i] = (long long)off;
+        if (ops[i].type == MLB_OP_GEMM) off += (size_t)(L / W2_NC) * W2_CL * (ops[i].Kpad < KS ? ops[i].Kpad : KS) * W2_NC;
+    }
+    cudaError_t e;
+    if ((e = cudaMalloc(&slab, off * sizeof(float))) != cudaSuccess) return e;
+    available = true;
+    if ((e = repack(blob, ops, n_ops, L, 0)) != cudaSuccess) return e;
+    if ((e = mlb_zalloc(&xg, (size_t)3 * L * W2_R * sizeof(unsigned long long))) != cudaSuccess) return e;
+    return mlb_zalloc(&hg, (size_t)(L / W2_NC) * W2_HQ * W2_R * sizeof(unsigned long long));
 }
 
-size_t mlb_wide2_xg_pairs(int L) { return (size_t)3 * L * W2_R; }
-size_t mlb_wide2_hg_pairs(int L) { return (size_t)(L / W2_NC) * W2_HQ * W2_R; }
+void Wide2Family::release() {
+    cudaFree(slab), cudaFree(xg), cudaFree(hg);
+    slab = nullptr, xg = nullptr, hg = nullptr;
+    available = false;
+}
 
-cudaError_t mlb_wide2_launch(const FwdParams& p, const float* wslab, const long long* wslab_off, unsigned long long* xg,
-                             unsigned long long* hg, unsigned epoch_base, cudaStream_t st) {
+cudaError_t Wide2Family::launch(FwdParams p, const FwdPlan&, cudaStream_t st, int* issued) {
     Wide2Extra ex;
-    ex.wslab = wslab;
-    for (int i = 0; i < MLB_MAX_OPS; ++i) ex.wslab_off[i] = i < p.n_ops ? wslab_off[i] : 0;
-    ex.xg = xg, ex.hg = hg, ex.epoch_base = epoch_base;
+    ex.wslab = slab;
+    for (int i = 0; i < MLB_MAX_OPS; ++i) ex.wslab_off[i] = i < p.n_ops ? slab_off[i] : 0;
+    ex.xg = xg, ex.hg = hg, ex.epoch_base = epoch;
+    p.n_tiles = 1, p.row_base = 0;
     // the opt-in shared-memory size is a per-function attribute of the PROCESS: another handle with a narrower model may have
     // lowered it since this one was created
     cudaError_t e = cudaFuncSetAttribute(loco_forward_wide2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wide2_smem(p.L));
@@ -470,5 +472,10 @@ cudaError_t mlb_wide2_launch(const FwdParams& p, const float* wslab, const long 
     at.id = cudaLaunchAttributeCooperative;   // co-residency of all clusters: they spin on each other's outputs
     at.val.cooperative = 1;
     cfg.attrs = &at, cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, loco_forward_wide2_kernel, p, ex);
+    if ((e = cudaLaunchKernelEx(&cfg, loco_forward_wide2_kernel, p, ex)) != cudaSuccess) return e;
+    unsigned n_epochs = 2;  // epochs one launch consumes
+    for (int i = 0; i < p.n_ops; ++i) n_epochs += p.ops[i].type == MLB_OP_GEMM;
+    epoch += n_epochs;
+    ++*issued;
+    return cudaSuccess;
 }

@@ -7,12 +7,8 @@
 #include <math.h>
 #include <stdint.h>
 
-#include <string>
-
 #include "../../include/monoloco_b200.h"
-
-extern thread_local std::string g_mlb_err;
-void mlb_count_launch();
+#include "host_error.h"
 
 namespace mlb {
 
@@ -82,10 +78,8 @@ extern "C" int mlb_adam_clip_step(int n_tensors, float* const* params, const flo
                                   float* const* exp_avg_sq, const int64_t* sizes, const int32_t* clip_mask, float max_norm,
                                   float lr, float beta1, float beta2, float eps, float weight_decay, int64_t step,
                                   double* sqnorm_scratch_dev, void* stream) {
-    if (n_tensors < 1 || !params || !grads || !exp_avg || !exp_avg_sq || !sizes || !sqnorm_scratch_dev || step < 1) {
-        g_mlb_err = "mlb_adam_clip_step: bad argument";
-        return -1;
-    }
+    if (n_tensors < 1 || !params || !grads || !exp_avg || !exp_avg_sq || !sizes || !sqnorm_scratch_dev || step < 1)
+        return mlb_fail("mlb_adam_clip_step: bad argument");
     cudaStream_t st = (cudaStream_t)stream;
     const float bc1 = 1.0f - powf(beta1, (float)step);
     const float bc2_sqrt = sqrtf(1.0f - powf(beta2, (float)step));
@@ -114,9 +108,6 @@ extern "C" int mlb_adam_clip_step(int n_tensors, float* const* params, const flo
         mlb_count_launch();
         e = cudaGetLastError();
     }
-    if (e != cudaSuccess) {
-        g_mlb_err = std::string("mlb_adam_clip_step: ") + cudaGetErrorString(e);
-        return -1;
-    }
+    if (e != cudaSuccess) return mlb_fail(std::string("mlb_adam_clip_step: ") + cudaGetErrorString(e));
     return 0;
 }

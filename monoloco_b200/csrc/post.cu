@@ -11,12 +11,8 @@
 #include <math.h>
 #include <stdint.h>
 
-#include <string>
-
 #include "../../include/monoloco_b200.h"
-
-extern thread_local std::string g_mlb_err;
-void mlb_count_launch();
+#include "host_error.h"
 
 namespace mlb {
 
@@ -245,45 +241,35 @@ __global__ void kitti_rows_kernel(int n, int out_size, double conf_scale, const 
 
 using namespace mlb;
 
-static int pfail(const std::string& msg) {
-    g_mlb_err = msg;
-    return -1;
-}
-#define PCU(call)                                                                                  \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess) return pfail(std::string(#call) + ": " + cudaGetErrorString(e_));  \
-    } while (0)
-
 extern "C" int mlb_stereo_filter(const float* raw, const float* dec, const float* xyzc, int n_left, int n_right, int out_size,
                                  float* sel_raw, float* sel_dec, float* sel_xyzc, int32_t* sel_idx, int32_t* n_sel_dev,
                                  int32_t* cnt_scratch, float* best_scratch, void* stream) {
     if (!raw || !sel_raw || !sel_idx || !n_sel_dev || !cnt_scratch || !best_scratch || n_left < 1 || n_right < 1 || out_size < 1)
-        return pfail("mlb_stereo_filter: bad argument");
+        return mlb_fail("mlb_stereo_filter: bad argument");
     const int wpb = 4, grid = (n_left + wpb - 1) / wpb;
     cudaStream_t st = (cudaStream_t)stream;
     stereo_count_kernel<<<grid, wpb * 32, 0, st>>>(raw, n_left, n_right, out_size, cnt_scratch, best_scratch);
     stereo_scatter_kernel<<<grid, wpb * 32, 0, st>>>(raw, dec, xyzc, n_left, n_right, out_size, cnt_scratch, best_scratch, sel_raw,
                                                      sel_dec, sel_xyzc, sel_idx, n_sel_dev);
-    PCU(cudaGetLastError());
+    MLB_CU(cudaGetLastError());
     mlb_count_launch();
     mlb_count_launch();
     return 0;
 }
 
 extern "C" int mlb_post_process(const mlb_post_args* a, void* stream) {
-    if (!a) return pfail("mlb_post_process: null argument");
-    if (a->n_img < 0 || a->max_det < 0 || a->max_gt < 0) return pfail("mlb_post_process: negative size");
+    if (!a) return mlb_fail("mlb_post_process: null argument");
+    if (a->n_img < 0 || a->max_det < 0 || a->max_gt < 0) return mlb_fail("mlb_post_process: negative size");
     if (a->n_img == 0) return 0;
     if (!a->det_off || !a->boxes || !a->kps || !a->kinv || !a->dec || !a->xyz || !a->ray || !a->conf || !a->uv || !a->match_gt ||
         !a->order || !a->n_match || !a->xyz_real)
-        return pfail("mlb_post_process: null pointer");
-    if (a->gt_off && (!a->gt_boxes || !a->gt_d)) return pfail("mlb_post_process: gt_off without gt_boxes / gt_d");
+        return mlb_fail("mlb_post_process: null pointer");
+    if (a->gt_off && (!a->gt_boxes || !a->gt_d)) return mlb_fail("mlb_post_process: gt_off without gt_boxes / gt_d");
     const size_t smem = ((size_t)3 * a->max_det + (size_t)a->max_gt + 4) * sizeof(int);
-    if (smem > 200 * 1024) return pfail("mlb_post_process: too many detections / ground truths in one image");
-    if (smem > 48 * 1024) PCU(cudaFuncSetAttribute(post_process_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem > 200 * 1024) return mlb_fail("mlb_post_process: too many detections / ground truths in one image");
+    if (smem > 48 * 1024) MLB_CU(cudaFuncSetAttribute(post_process_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     post_process_kernel<<<a->n_img, 128, smem, (cudaStream_t)stream>>>(*a);
-    PCU(cudaGetLastError());
+    MLB_CU(cudaGetLastError());
     mlb_count_launch();
     return 0;
 }
@@ -291,9 +277,9 @@ extern "C" int mlb_post_process(const mlb_post_args* a, void* stream) {
 extern "C" int mlb_kitti_rows(int n, int out_size, double conf_scale, const double* boxes, const float* raw, const float* dec,
                               const float* epi, double* rows, void* stream) {
     if (n == 0) return 0;
-    if (n < 0 || out_size < 7 || !boxes || !raw || !dec || !rows) return pfail("mlb_kitti_rows: bad argument");
+    if (n < 0 || out_size < 7 || !boxes || !raw || !dec || !rows) return mlb_fail("mlb_kitti_rows: bad argument");
     kitti_rows_kernel<<<(n + 127) / 128, 128, 0, (cudaStream_t)stream>>>(n, out_size, conf_scale, boxes, raw, dec, epi, rows);
-    PCU(cudaGetLastError());
+    MLB_CU(cudaGetLastError());
     mlb_count_launch();
     return 0;
 }

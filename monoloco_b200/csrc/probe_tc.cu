@@ -15,9 +15,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#include <string>
-
 #include "common.cuh"
+#include "host_error.h"
 
 namespace mlb {
 
@@ -260,26 +259,18 @@ __global__ void __launch_bounds__(128, 1) tc_layer_kernel(const float* __restric
 
 }  // namespace mlb
 
-extern thread_local std::string g_mlb_err;
-void mlb_count_launch();
-
 extern "C" int mlb_probe_tf32x3(const float* A_dev, const float* W_dev, int K, int mode, float* out_main_dev, float* out_cross_dev,
                                 void* stream) {
     using namespace mlb;
-    if (!A_dev || !W_dev || !out_main_dev || K < PKB || (K % PKB) != 0 || mode < 0 || mode > 2) {
-        g_mlb_err = "mlb_probe_tf32x3: A [128,K], W [128,K] (K a multiple of 32), out [128,128], mode 0..2";
-        return -1;
-    }
+    if (!A_dev || !W_dev || !out_main_dev || K < PKB || (K % PKB) != 0 || mode < 0 || mode > 2)
+        return mlb_fail("mlb_probe_tf32x3: A [128,K], W [128,K] (K a multiple of 32), out [128,128], mode 0..2");
     const size_t smem = (size_t)(2 * PM + 2 * PN) * PKB * sizeof(float);
     cudaError_t e = cudaFuncSetAttribute(tc_probe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e == cudaSuccess) {
         tc_probe_kernel<<<1, 128, smem, (cudaStream_t)stream>>>(A_dev, W_dev, K, mode, out_main_dev, out_cross_dev, nullptr);
         e = cudaGetLastError();
     }
-    if (e != cudaSuccess) {
-        g_mlb_err = std::string("mlb_probe_tf32x3: ") + cudaGetErrorString(e);
-        return -1;
-    }
+    if (e != cudaSuccess) return mlb_fail(std::string("mlb_probe_tf32x3: ") + cudaGetErrorString(e));
     mlb_count_launch();
     return 0;
 }
@@ -289,10 +280,8 @@ extern "C" int mlb_probe_tf32x3(const float* A_dev, const float* W_dev, int K, i
 extern "C" int mlb_probe_tc_layer(const float* X_dev, const float* W_dev, float* Y_dev, int B, int N, int K, float* x_planes_dev,
                                   float* w_planes_dev, int stages, void* stream) {
     using namespace mlb;
-    if (!x_planes_dev || !w_planes_dev || B < LM || (B % LM) || N < LN || (N % LN) || K < LKB || (K % LKB)) {
-        g_mlb_err = "mlb_probe_tc_layer: B % 128 == 0, N % 256 == 0, K % 16 == 0 and both plane buffers are required";
-        return -1;
-    }
+    if (!x_planes_dev || !w_planes_dev || B < LM || (B % LM) || N < LN || (N % LN) || K < LKB || (K % LKB))
+        return mlb_fail("mlb_probe_tc_layer: B % 128 == 0, N % 256 == 0, K % 16 == 0 and both plane buffers are required");
     cudaStream_t st = (cudaStream_t)stream;
     cudaError_t e = cudaSuccess;
     if ((stages & 1) && X_dev) tc_pack_planes_kernel<<<296, 256, 0, st>>>(X_dev, x_planes_dev, B, K, LM), mlb_count_launch();
@@ -306,9 +295,6 @@ extern "C" int mlb_probe_tc_layer(const float* X_dev, const float* W_dev, float*
         }
     }
     if (e == cudaSuccess) e = cudaGetLastError();
-    if (e != cudaSuccess) {
-        g_mlb_err = std::string("mlb_probe_tc_layer: ") + cudaGetErrorString(e);
-        return -1;
-    }
+    if (e != cudaSuccess) return mlb_fail(std::string("mlb_probe_tc_layer: ") + cudaGetErrorString(e));
     return 0;
 }

@@ -26,9 +26,8 @@
 #include <stdint.h>
 #include <string.h>
 
-#include <string>
-
 #include "gemm_tile.cuh"
+#include "host_error.h"
 
 namespace mlb {
 
@@ -928,19 +927,6 @@ struct mlb_train {
     int last_phase_type[MAX_PHASES], last_phase_blk[MAX_PHASES];
 };
 
-extern thread_local std::string g_mlb_err;
-static int tfail(const std::string& m) {
-    g_mlb_err = m;
-    return -1;
-}
-#define TCU(call)                                                                                  \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess) return tfail(std::string(#call) + ": " + cudaGetErrorString(e_));  \
-    } while (0)
-
-void mlb_count_launch();
-
 static size_t train_smem_bytes(int L) {
     size_t actf = (size_t)L * MP > 8 * 32 * 33 ? (size_t)L * MP : 8 * 32 * 33;
     size_t fl = actf + MP * OUT_LD + (size_t)NSTAGE * KC * L;
@@ -948,13 +934,13 @@ static size_t train_smem_bytes(int L) {
 }
 
 extern "C" int mlb_train_create(int device, int max_rows, int input_size, int linear_size, int n_blocks, mlb_train_handle* out) {
-    if (!out || max_rows < 2 || n_blocks < 2 || n_blocks > MLB_MAX_BLOCKS) return tfail("mlb_train_create: bad argument");
-    if (linear_size < 128 || linear_size > 1024 || linear_size % 128) return tfail("mlb_train_create: linear_size must be a multiple of 128 in [128,1024]");
-    if (input_size < 1 || input_size > 68) return tfail("mlb_train_create: input_size must be in [1,68]");
-    TCU(cudaSetDevice(device));
+    if (!out || max_rows < 2 || n_blocks < 2 || n_blocks > MLB_MAX_BLOCKS) return mlb_fail("mlb_train_create: bad argument");
+    if (linear_size < 128 || linear_size > 1024 || linear_size % 128) return mlb_fail("mlb_train_create: linear_size must be a multiple of 128 in [128,1024]");
+    if (input_size < 1 || input_size > 68) return mlb_fail("mlb_train_create: input_size must be in [1,68]");
+    MLB_CU(cudaSetDevice(device));
     cudaDeviceProp prop;
-    TCU(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) return tfail("mlb_train_create: built for sm_100a (B200) only");
+    MLB_CU(cudaGetDeviceProperties(&prop, device));
+    if (prop.major != 10) return mlb_fail("mlb_train_create: built for sm_100a (B200) only");
     mlb_train* t = new mlb_train();
     memset(t, 0, sizeof(*t));
     t->device = device, t->n_sms = prop.multiProcessorCount, t->max_rows = max_rows, t->in_size = input_size;
@@ -963,27 +949,27 @@ extern "C" int mlb_train_create(int device, int max_rows, int input_size, int li
     const size_t act_bytes = (size_t)t->rows_pad * linear_size * sizeof(float);
     for (int i = 0; i < n_blocks; ++i) {
         const int kpad = i == 0 ? ((input_size + KC - 1) / KC) * KC : linear_size;
-        TCU(cudaMalloc(&t->Wt[i], (size_t)kpad * linear_size * sizeof(float)));
-        TCU(cudaMalloc(&t->Z[i], act_bytes));
-        TCU(cudaMalloc(&t->A[i], act_bytes));
-        TCU(cudaMalloc(&t->G[i], act_bytes));
-        TCU(cudaMalloc(&t->Gz[i], act_bytes));
-        TCU(cudaMemset(t->Z[i], 0, act_bytes));
-        TCU(cudaMemset(t->A[i], 0, act_bytes));
-        TCU(cudaMemset(t->G[i], 0, act_bytes));
-        TCU(cudaMemset(t->Gz[i], 0, act_bytes));
-        TCU(cudaMalloc(&t->stat[i], 4 * linear_size * sizeof(double)));
-        TCU(cudaMemset(t->stat[i], 0, 4 * linear_size * sizeof(double)));
+        MLB_CU(cudaMalloc(&t->Wt[i], (size_t)kpad * linear_size * sizeof(float)));
+        MLB_CU(cudaMalloc(&t->Z[i], act_bytes));
+        MLB_CU(cudaMalloc(&t->A[i], act_bytes));
+        MLB_CU(cudaMalloc(&t->G[i], act_bytes));
+        MLB_CU(cudaMalloc(&t->Gz[i], act_bytes));
+        MLB_CU(cudaMemset(t->Z[i], 0, act_bytes));
+        MLB_CU(cudaMemset(t->A[i], 0, act_bytes));
+        MLB_CU(cudaMemset(t->G[i], 0, act_bytes));
+        MLB_CU(cudaMemset(t->Gz[i], 0, act_bytes));
+        MLB_CU(cudaMalloc(&t->stat[i], 4 * linear_size * sizeof(double)));
+        MLB_CU(cudaMemset(t->stat[i], 0, 4 * linear_size * sizeof(double)));
     }
-    TCU(cudaMalloc(&t->g_out, (size_t)t->rows_pad * OUT_LD * sizeof(float)));
-    TCU(cudaMemset(t->g_out, 0, (size_t)t->rows_pad * OUT_LD * sizeof(float)));
-    TCU(cudaMalloc(&t->loss_acc, 8 * sizeof(double)));
-    TCU(cudaMalloc(&t->ptab, (size_t)t->n_sms * linear_size * 2 * sizeof(float4)));
-    TCU(cudaMalloc(&t->bar, sizeof(unsigned)));
-    TCU(cudaMalloc(&t->err, sizeof(int)));
-    TCU(cudaMemset(t->err, 0, sizeof(int)));
-    TCU(cudaMalloc(&t->phase_ns, (MAX_PHASES + 1 + MAX_PHASES * 24) * sizeof(unsigned long long)));
-    TCU(cudaMemset(t->phase_ns, 0, (MAX_PHASES + 1 + MAX_PHASES * 24) * sizeof(unsigned long long)));
+    MLB_CU(cudaMalloc(&t->g_out, (size_t)t->rows_pad * OUT_LD * sizeof(float)));
+    MLB_CU(cudaMemset(t->g_out, 0, (size_t)t->rows_pad * OUT_LD * sizeof(float)));
+    MLB_CU(cudaMalloc(&t->loss_acc, 8 * sizeof(double)));
+    MLB_CU(cudaMalloc(&t->ptab, (size_t)t->n_sms * linear_size * 2 * sizeof(float4)));
+    MLB_CU(cudaMalloc(&t->bar, sizeof(unsigned)));
+    MLB_CU(cudaMalloc(&t->err, sizeof(int)));
+    MLB_CU(cudaMemset(t->err, 0, sizeof(int)));
+    MLB_CU(cudaMalloc(&t->phase_ns, (MAX_PHASES + 1 + MAX_PHASES * 24) * sizeof(unsigned long long)));
+    MLB_CU(cudaMemset(t->phase_ns, 0, (MAX_PHASES + 1 + MAX_PHASES * 24) * sizeof(unsigned long long)));
     *out = t;
     return 0;
 }
@@ -1019,17 +1005,17 @@ static int pick_tm(int n_rows, int n_ctas) {
 
 // mode: 0 forward, 1 backward, 2 fused step
 static int train_launch(mlb_train_handle t, const mlb_train_args* a, const mlb_train_block* blocks, void* stream, int mode) {
-    if (!t || !a || !blocks) return tfail("mlb_train: null argument");
-    if (a->n_rows < 2 || a->n_rows > t->max_rows) return tfail("mlb_train: n_rows must be in [2, max_rows] (BatchNorm needs > 1 row)");
-    if (a->linear_size != t->L || a->n_blocks != t->n_blocks || a->input_size != t->in_size) return tfail("mlb_train: shape differs from mlb_train_create");
-    if (a->output_size < 2 || a->output_size > OUT_LD) return tfail("mlb_train: bad output_size");
-    if (a->aux_block < 0 || a->aux_block >= a->n_blocks - 1) return tfail("mlb_train: bad aux_block");
-    if (!a->x || !a->out || !a->W_aux || !a->b_aux || !a->W_fin || !a->b_fin) return tfail("mlb_train: missing tensor");
-    if (mode >= 1 && (!a->dW_aux || !a->db_aux || !a->dW_fin || !a->db_fin)) return tfail("mlb_train: missing head gradient buffers");
-    if (mode == 1 && !a->g_out) return tfail("mlb_train_backward: g_out required");
-    if (mode == 2 && (!a->labels || !a->loss_vals || a->n_tasks < 1 || a->n_tasks > 8)) return tfail("mlb_train_step: labels / loss_vals / tasks required");
-    if (a->p_dropout < 0.f || a->p_dropout >= 1.f) return tfail("mlb_train: bad p_dropout");
-    TCU(cudaSetDevice(t->device));
+    if (!t || !a || !blocks) return mlb_fail("mlb_train: null argument");
+    if (a->n_rows < 2 || a->n_rows > t->max_rows) return mlb_fail("mlb_train: n_rows must be in [2, max_rows] (BatchNorm needs > 1 row)");
+    if (a->linear_size != t->L || a->n_blocks != t->n_blocks || a->input_size != t->in_size) return mlb_fail("mlb_train: shape differs from mlb_train_create");
+    if (a->output_size < 2 || a->output_size > OUT_LD) return mlb_fail("mlb_train: bad output_size");
+    if (a->aux_block < 0 || a->aux_block >= a->n_blocks - 1) return mlb_fail("mlb_train: bad aux_block");
+    if (!a->x || !a->out || !a->W_aux || !a->b_aux || !a->W_fin || !a->b_fin) return mlb_fail("mlb_train: missing tensor");
+    if (mode >= 1 && (!a->dW_aux || !a->db_aux || !a->dW_fin || !a->db_fin)) return mlb_fail("mlb_train: missing head gradient buffers");
+    if (mode == 1 && !a->g_out) return mlb_fail("mlb_train_backward: g_out required");
+    if (mode == 2 && (!a->labels || !a->loss_vals || a->n_tasks < 1 || a->n_tasks > 8)) return mlb_fail("mlb_train_step: labels / loss_vals / tasks required");
+    if (a->p_dropout < 0.f || a->p_dropout >= 1.f) return mlb_fail("mlb_train: bad p_dropout");
+    MLB_CU(cudaSetDevice(t->device));
     cudaStream_t st = (cudaStream_t)stream;
 
     TrainParams p;
@@ -1038,11 +1024,11 @@ static int train_launch(mlb_train_handle t, const mlb_train_args* a, const mlb_t
     for (int i = 0; i < a->n_blocks; ++i) {
         const mlb_train_block& s = blocks[i];
         TBlk& b = p.blk[i];
-        if (s.K != (i == 0 ? a->input_size : a->linear_size)) return tfail("mlb_train: block K mismatch");
-        if (!s.W || !s.b || (s.has_bn && (!s.gamma || !s.beta))) return tfail("mlb_train: missing block parameter");
-        if (mode >= 1 && (!s.dW || !s.db || (s.has_bn && (!s.dgamma || !s.dbeta)))) return tfail("mlb_train: missing block gradient buffer");
-        if (i == 0 && !s.has_bn) return tfail("mlb_train: the first block must have BatchNorm");
-        if (s.res_src >= i) return tfail("mlb_train: bad res_src");
+        if (s.K != (i == 0 ? a->input_size : a->linear_size)) return mlb_fail("mlb_train: block K mismatch");
+        if (!s.W || !s.b || (s.has_bn && (!s.gamma || !s.beta))) return mlb_fail("mlb_train: missing block parameter");
+        if (mode >= 1 && (!s.dW || !s.db || (s.has_bn && (!s.dgamma || !s.dbeta)))) return mlb_fail("mlb_train: missing block gradient buffer");
+        if (i == 0 && !s.has_bn) return mlb_fail("mlb_train: the first block must have BatchNorm");
+        if (s.res_src >= i) return mlb_fail("mlb_train: bad res_src");
         b.K = s.K;
         b.Kpad = ((s.K + KC - 1) / KC) * KC;
         b.has_bn = s.has_bn;
@@ -1056,13 +1042,13 @@ static int train_launch(mlb_train_handle t, const mlb_train_args* a, const mlb_t
     }
     for (int i = 0; i < a->n_blocks; ++i)
         if (p.blk[i].res_src >= 0) p.blk[p.blk[i].res_src].skip_to = i;
-    if (!p.blk[a->n_blocks - 1].has_bn) return tfail("mlb_train: the last block must have BatchNorm (LocoModel.w3)");
-    if (p.blk[a->aux_block].has_bn) return tfail("mlb_train: aux_block must be the BatchNorm-free block (LocoModel.w2)");
+    if (!p.blk[a->n_blocks - 1].has_bn) return mlb_fail("mlb_train: the last block must have BatchNorm (LocoModel.w3)");
+    if (p.blk[a->aux_block].has_bn) return mlb_fail("mlb_train: aux_block must be the BatchNorm-free block (LocoModel.w2)");
     p.n_blocks = a->n_blocks, p.aux_block = a->aux_block, p.L = a->linear_size, p.in_size = a->input_size;
     p.out_size = a->output_size, p.n_rows = a->n_rows;
     p.n_rows_pad = ((a->n_rows + KC - 1) / KC) * KC;
     int tm = a->rows_per_group ? a->rows_per_group : pick_tm(a->n_rows, t->n_sms);
-    if (tm < 8 || tm > 16 || (tm & 1)) return tfail("mlb_train: rows_per_group must be 0 or one of 8,10,12,14,16");
+    if (tm < 8 || tm > 16 || (tm & 1)) return mlb_fail("mlb_train: rows_per_group must be 0 or one of 8,10,12,14,16");
     p.n_tiles = (a->n_rows + 2 * tm - 1) / (2 * tm);
     p.p_drop = a->p_dropout, p.eps = a->bn_eps > 0.f ? a->bn_eps : 1e-5f, p.momentum = a->bn_momentum;
     p.update_running = a->update_running_stats;
@@ -1073,8 +1059,8 @@ static int train_launch(mlb_train_handle t, const mlb_train_args* a, const mlb_t
     if (mode == 2) {
         p.labels = a->labels, p.label_ld = a->label_ld, p.n_tasks = a->n_tasks;
         for (int i = 0; i < a->n_tasks; ++i) {
-            if (a->tasks[i] < 0 || a->tasks[i] > MLB_TASK_AUX) return tfail("mlb_train_step: bad task id");
-            if (a->tasks[i] == MLB_TASK_AUX && (a->output_size != 10 || a->label_ld < 11)) return tfail("mlb_train_step: aux task needs 10 outputs / 11 label columns");
+            if (a->tasks[i] < 0 || a->tasks[i] > MLB_TASK_AUX) return mlb_fail("mlb_train_step: bad task id");
+            if (a->tasks[i] == MLB_TASK_AUX && (a->output_size != 10 || a->label_ld < 11)) return mlb_fail("mlb_train_step: aux task needs 10 outputs / 11 label columns");
             p.tasks[i] = a->tasks[i], p.task_scale[i] = a->task_scale[i];
         }
         p.loss_vals = a->loss_vals;
@@ -1098,12 +1084,12 @@ static int train_launch(mlb_train_handle t, const mlb_train_args* a, const mlb_t
         add(PH_DW, 0);
     }
     p.n_phases = np;
-    if (np > MAX_PHASES) return tfail("mlb_train: too many phases");
+    if (np > MAX_PHASES) return mlb_fail("mlb_train: too many phases");
     t->last_n_phases = np;
     memcpy(t->last_phase_type, p.phase_type, sizeof(int) * np);
     memcpy(t->last_phase_blk, p.phase_blk, sizeof(int) * np);
 
-    TCU(cudaMemsetAsync(t->bar, 0, sizeof(unsigned), st));
+    MLB_CU(cudaMemsetAsync(t->bar, 0, sizeof(unsigned), st));
     const size_t smem = train_smem_bytes(a->linear_size);
     const int grid = t->n_sms;
     cudaError_t e;
@@ -1114,18 +1100,18 @@ static int train_launch(mlb_train_handle t, const mlb_train_args* a, const mlb_t
         case 14: e = launch_train<14>(p, grid, smem, st); break;
         default: e = launch_train<16>(p, grid, smem, st); break;
     }
-    if (e != cudaSuccess) return tfail(std::string("loco_train_kernel launch: ") + cudaGetErrorString(e));
+    if (e != cudaSuccess) return mlb_fail(std::string("loco_train_kernel launch: ") + cudaGetErrorString(e));
     mlb_count_launch();
     return 0;
 }
 
 // per-phase wall time (ns) of the most recent launch on this handle: out_ns[i] = duration of phase i, types/blks describe it
 extern "C" int mlb_train_phase_times(mlb_train_handle t, int max_n, double* out_ns, int* types, int* blks) {
-    if (!t || !out_ns) return tfail("mlb_train_phase_times: bad argument");
-    TCU(cudaSetDevice(t->device));
-    TCU(cudaDeviceSynchronize());
+    if (!t || !out_ns) return mlb_fail("mlb_train_phase_times: bad argument");
+    MLB_CU(cudaSetDevice(t->device));
+    MLB_CU(cudaDeviceSynchronize());
     unsigned long long ts[MAX_PHASES + 1];
-    TCU(cudaMemcpy(ts, t->phase_ns, sizeof(ts), cudaMemcpyDeviceToHost));
+    MLB_CU(cudaMemcpy(ts, t->phase_ns, sizeof(ts), cudaMemcpyDeviceToHost));
     int n = t->last_n_phases < max_n ? t->last_n_phases : max_n;
     for (int i = 0; i < n; ++i) {
         out_ns[i] = (double)(ts[i + 1] - ts[i]);
@@ -1138,11 +1124,11 @@ extern "C" int mlb_train_phase_times(mlb_train_handle t, int max_n, double* out_
 // profiling aid: out_ns[(ph*3 + s)*8 + k] = time since the start of phase ph at which CTA s (0: first, 1: middle, 2: last
 // active) passed point k (0: input tile ready, 1: GEMM done, 2: epilogue done, 3: left the grid barrier, 4 batch statistics loaded, 5 tile rows finished, 6-7 spare); 0 where unset.
 extern "C" int mlb_train_subphase_times(mlb_train_handle t, int max_n, double* out_ns) {
-    if (!t || !out_ns) return tfail("mlb_train_subphase_times: bad argument");
-    TCU(cudaSetDevice(t->device));
-    TCU(cudaDeviceSynchronize());
+    if (!t || !out_ns) return mlb_fail("mlb_train_subphase_times: bad argument");
+    MLB_CU(cudaSetDevice(t->device));
+    MLB_CU(cudaDeviceSynchronize());
     static unsigned long long ts[MAX_PHASES + 1 + MAX_PHASES * 24];
-    TCU(cudaMemcpy(ts, t->phase_ns, sizeof(ts), cudaMemcpyDeviceToHost));
+    MLB_CU(cudaMemcpy(ts, t->phase_ns, sizeof(ts), cudaMemcpyDeviceToHost));
     int n = t->last_n_phases < max_n ? t->last_n_phases : max_n;
     for (int i = 0; i < n; ++i)
         for (int q = 0; q < 24; ++q) {
